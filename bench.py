@@ -178,6 +178,25 @@ def pinned_uniform(shape, seed):
     return t, a
 
 
+DUMP_BYTES = 60 << 20    # --dump-outputs stays below 64 MB in all
+
+
+def dump_outputs(out_dir, eng, n, r, last, write=True):
+    """--dump-outputs: what the timed loop leaves its caller after its last step, as float64 .npy files in out_dir -- the
+    iterate R, the gradient G and the multipliers lambda (vertex / constraint order of the input) at a fixed, seeded
+    sample of the vertices (MaxCut has one constraint per vertex), the sampled indices, and (L, obj, ||G||^2, ||pvio||^2,
+    alpha) of the last step.  Same arguments, same files: two builds can be compared output for output.  With several
+    ranks every rank must call this (the downloads gather over all of them); only the one with write=True writes."""
+    k = min(n, 1 << 18, DUMP_BYTES // (8 * (2 * r + 2)))
+    rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    arrays = {"rows": rows, "R": eng.get_R()[rows], "G": eng.get_G()[rows], "lambda": eng.get_lambda()[rows],
+              "last_iterate": np.asarray(last)}
+    if write:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def host_threads():
     """Host threads the CPU arm may use: the affinity mask, not OMP_NUM_THREADS (torchrun exports OMP_NUM_THREADS=1)."""
     try:
@@ -186,7 +205,7 @@ def host_threads():
         return max(1, os.cpu_count() or 1)
 
 
-def cpu_oracle_run(sp, n, edges, r, steps, warmup, seed, single_thread_steps=1, budget_s=150.0, adopt=None):
+def cpu_oracle_run(sp, n, edges, r, steps, warmup, seed, single_thread_steps=1, budget_s=150.0, adopt=None, dump_dir=None):
     """The reference's CPU path (oracle port of src/*.jl) on the SAME workload as the GPU arm: the same graph
     (same generator, same seed, same n and edge count), the same R0, the same loop body.  Timed twice:
     with all host threads (OpenMP; the thread count is set here, whatever the launcher exported) and with ONE
@@ -230,6 +249,8 @@ def cpu_oracle_run(sp, n, edges, r, steps, warmup, seed, single_thread_steps=1, 
     last = sp.solver.run_inner_iterations(eng, k)
     dt = time.perf_counter() - t0
     its = k / dt
+    if dump_dir:
+        dump_outputs(dump_dir, eng, n, r, last)
     single = None
     if single_thread_steps > 0 and cores > 1:
         lib.orc_set_threads(1)
@@ -275,6 +296,8 @@ def main():
     ap.add_argument("--solve-maxtime", type=float, default=240.0, help="time limit of the time-to-tolerance solve in seconds")
     ap.add_argument("--host-triplets", action="store_true", help="hand the problem to sdplrp_preprocess as HOST triplets (4.4 GB D2H + H2D per "
                     "rank) instead of keeping the generator's triplets on the device (sdplrp_preprocess_device); affects the setup times only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what they computed as DIR/<name>.npy "
+                    "(float64, a fixed sample of the rows; see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -288,7 +311,7 @@ def main():
         if rank != 0:
             return 0
         res = cpu_oracle_run(sp, args.n, args.edges, args.rank, min(args.steps, args.cpu_steps), min(args.warmup, 2), args.seed,
-                             single_thread_steps=args.cpu_single_steps, budget_s=args.cpu_budget_s)
+                             single_thread_steps=args.cpu_single_steps, budget_s=args.cpu_budget_s, dump_dir=args.dump_outputs)
         line = {"impl": "reference", "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": res["steps"],
                 "warmup": res["warmup"], "requested_steps": args.steps, "requested_warmup": args.warmup,
                 "ms_per_step": res["ms_per_iter"], "higher_is_better": True, "scaling": "strong",
@@ -369,6 +392,8 @@ def main():
     dev_ms = spdist.max_over_ranks(dev_ms)
     t_wall = spdist.max_over_ranks(t_wall)
     value = args.steps / (dev_ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, n, r, last, write=rank == 0)
 
     # ---- end to end through the public API with host buffers: upload R0/lambda0 from pinned
     #      memory, K iterations (host scalars cross every iteration), download R/lambda

@@ -1,14 +1,10 @@
 """On-disk formats (SURVEY.md 8f/f4): the SDPA / SDPLR-1.03 writers of exps/data_utils.jl:22-152 restated in
-sdplrplus.jl_b200/formats.py, their readers (round trips), the Gset reader and the MATLAB v7.3 reader."""
-import os
-
+sdplrplus.jl_b200/formats.py, their readers (round trips) and the Gset reader."""
 import numpy as np
 import pytest
 import scipy.sparse as sps
 
 from helpers import g1_graph, k2_graph, p3_graph
-
-REF_DATA = "/root/reference/exps/data"
 
 
 @pytest.fixture(scope="module")
@@ -114,15 +110,3 @@ def test_gset_reader(F, tmp_path):
     G = g1_graph()
     F.write_gset(tmp_path / "g1.txt", G)
     assert (F.read_graph(tmp_path / "g1.txt") != G).nnz == 0
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="the reference's data files exist only in the build container")
-def test_mat_v73_reader_on_the_reference_files(F):
-    G = g1_graph()
-    for fam in ("MaxCut", "LovaszTheta", "MinimumBisection", "CutNorm"):
-        A = F.read_graph(os.path.join(REF_DATA, fam, "G1.mat"))
-        assert (A != G).nnz == 0
-    A6 = F.read_mat_sparse(os.path.join(REF_DATA, "CutNorm", "G6.mat"), "A")
-    assert A6.shape == (800, 800) and A6.nnz == 38352 and set(np.unique(A6.data)) == {-1.0, 1.0} and abs(A6 - A6.T).max() == 0
-    with pytest.raises(KeyError):
-        F.read_mat_sparse(os.path.join(REF_DATA, "MaxCut", "G1.mat"), "B")

@@ -1,6 +1,6 @@
 """julia/SDPLRPlusB200.jl cannot be executed here (no Julia toolchain).  What CAN be pinned without one: every `ccall` of the
 shim names an entry point that include/sdplrp_b200.h declares, with the same number of arguments and compatible scalar
-types, and every reference function the shim adds a method to is imported from SDPLRPlus by name."""
+types, and the shim's mirrors of the native structs match the header field for field."""
 import os
 import re
 
@@ -96,15 +96,3 @@ def test_mode_fields_are_compared_as_symbols():
     jl = open(os.path.join(ROOT, "julia", "SDPLRPlusB200.jl")).read()
     assert '== "relative"' not in jl
     assert jl.count("== :relative") >= 5
-
-
-def test_overloaded_reference_functions_exist():
-    ref = "/root/reference/src"
-    if not os.path.isdir(ref):
-        import pytest
-        pytest.skip("reference checkout not mounted (GPU box)")
-    text = "".join(open(os.path.join(ref, f)).read() for f in os.listdir(ref) if f.endswith(".jl"))
-    jl = open(os.path.join(ROOT, "julia", "SDPLRPlusB200.jl")).read()
-    imported = re.search(r"import SDPLRPlus: (.*?)\n\n", jl, flags=re.S).group(1).replace("\n", " ")
-    for name in [x.strip() for x in imported.split(",")]:
-        assert re.search(r"(function |struct |^)" + re.escape(name) + r"(?![\w!])", text, flags=re.M), f"{name} not found in the reference sources"
