@@ -274,6 +274,18 @@ int32_t sdplrp_dimacs_errors(sdplrp_handle *h, double normb, double normC, const
 /* host helper: eigen-decomposition of a small dense symmetric matrix A (k x k row-major): ascending eigenvalues ev[k],
  * eigenvectors as the columns of Q (k x k row-major, may be NULL).  The projected problem of the restarted Lanczos. */
 int32_t sdplrp_dense_symeig(const double *A, int64_t k, double *ev, double *Q);
+/* Hyperplane rounding (Goemans-Williamson) of the current R: K candidates x_k = sign(R g_k), x_{k,i} = +1 when
+ * <R_i, g_k> >= 0, else -1.  g_k in R^r: rows of G (K x r row-major, host) or, G NULL, standard normals from a
+ * counter-based generator keyed by (seed, k, column) -- the same hyperplanes for every GPU count, vertex order and
+ * K (candidate k of a call with K = 100 equals candidate k of a call with K = 64).  G_out (K x r, may be NULL) receives
+ * the hyperplanes used.  obj[k] = <C, x_k x_k'> over the sparse objective (the quantity sdplrp_get_obj reports for R),
+ * sum[k] = sum_i x_{k,i} (may be NULL; the imbalance of a bisection).  best (1-based) is the candidate with the smallest
+ * obj, ties to the lowest k; best_x (n, host, reference vertex order, may be NULL) receives it as +-1.0.
+ * Reads R only: no other device state (G, D, CR, CD, y, S, residuals, L-BFGS history, W0/W1) changes.
+ * Several GPUs: every rank passes the same K, seed and G and receives the same results.
+ * SDPLRP_ERR_ARG for K < 1, NULL obj / best, and when C has a low-rank part (or no sparse part). */
+int32_t sdplrp_round_hyperplane(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, double *G_out,
+                                double *obj, double *sum, int64_t *best, double *best_x);
 
 /* ---- native host driver (SURVEY.md 8f, f1) ------------------------------ */
 /* BurerMonteiroConfig (src/options.jl:1-24); every field is 8 bytes wide so the layout is the same from C, Julia

@@ -354,6 +354,23 @@ function SDPLRPlus.DIMACS_errors(data, var::SolverVars{Ti,Float64,DevMat}, aux::
     return errs
 end
 
+"""
+    round_hyperplane(aux, K; r, G = nothing, seed = 0) -> (obj, sum, best, best_x, G_used)
+
+Goemans-Williamson rounding of the current R (rank `r`) on the device: K candidates x_k = sign(R' g_k) (+1 on ties),
+obj[k] = <C, x_k x_k'>, sum[k] = sum(x_k), `best` (1-based) the smallest obj, `best_x` its +-1 vector.  `G` (r x K, one
+hyperplane per column) or, `nothing`, seeded standard normals (the same for every K and GPU count).  Reads R only.
+"""
+function round_hyperplane(aux::B200Auxiliary, K::Integer; r::Integer, G=nothing, seed=0)
+    Gin = G === nothing ? Ptr{Float64}(C_NULL) : Matrix{Float64}(G)
+    G === nothing || size(Gin) == (r, K) || throw(ArgumentError("G must be r x K"))
+    G_used = zeros(r, K); obj = zeros(K); tot = zeros(K); best = Ref{Int64}(0); x = zeros(aux.n)
+    GC.@preserve Gin G_used obj tot x check(aux.h, ccall((:sdplrp_round_hyperplane, LIB), Int32,
+        (Ptr{Cvoid}, Int64, Ptr{Float64}, UInt64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Int64}, Ptr{Float64}),
+        aux.h.ptr, K, Gin, UInt64(seed), G_used, obj, tot, best, x))
+    return obj, tot, Int(best[]), x, G_used
+end
+
 function apply_kwargs!(config, kwargs)
     for (k, v) in kwargs
         hasfield(BurerMonteiroConfig, Symbol(k)) ? setfield!(config, Symbol(k), v) : @error "Unrecognized keyword argument $k"
@@ -381,6 +398,7 @@ function sdplr(C::AbstractMatrix{Float64}, As::Vector, b::Vector{Float64}, r::In
     ans["Rt"] = Array(ans["Rt"])                 # the reference returns host matrices
     ans["preprocess_time"] = preprocess_dt
     ans["totaltime"] += preprocess_dt
+    ans["aux"] = aux                             # R stays on the device: round_hyperplane(ans["aux"], K; r = ans["r"])
     return ans
 end
 
@@ -429,7 +447,7 @@ function sdplr_native(C::AbstractMatrix{Float64}, As::Vector, b::Vector{Float64}
         "primal_vio" => R.primal_vio, "obj" => R.obj, "max_dual_value" => R.max_dual_value, "min_duality_gap" => R.min_duality_gap,
         "totaltime" => R.totaltime, "dual_time" => R.dual_time, "primaltime" => R.primaltime, "iter" => R.iter,
         "majoriter" => R.majoriter, "DIMACS_errs" => collect(R.DIMACS_errs), "ptol" => config.ptol, "objtol" => config.objtol,
-        "fprec" => config.fprec, "rankupd_tol" => config.rankupd_tol, "r" => Int(R.r))
+        "fprec" => config.fprec, "rankupd_tol" => config.rankupd_tol, "r" => Int(R.r), "aux" => aux)
 end
 
 end # module

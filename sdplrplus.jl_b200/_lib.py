@@ -114,6 +114,7 @@ _SIGNATURES.update({
     "sdplrp_pick_alpha": [_p_f64, C.c_double, _p_f64, _p_f64],
     "sdplrp_iterate": [_H, C.c_int64, C.c_double, C.c_int32, C.c_int32, _p_f64],
     "sdplrp_fill_uniform": [_H, C.c_int32, C.c_uint64],
+    "sdplrp_round_hyperplane": [_H, C.c_int64, _p_f64, C.c_uint64, _p_f64, _p_f64, _p_f64, _p_i64, _p_f64],
 })
 
 _SPECIAL = {
@@ -519,6 +520,21 @@ class Handle:
     def fill_uniform(self, mat_id, seed):
         """mat <- U(-1,1) from the counter-based device generator (same matrix for any GPU count / vertex order)"""
         self._check(self.lib.sdplrp_fill_uniform(self._h, int(mat_id), int(seed)))
+
+    def round_hyperplane(self, K, G=None, seed=0):
+        """sdplrp_round_hyperplane: K hyperplane roundings x_k = sign(R g_k) of the current R ->
+        dict(obj (K,), sum (K,), best (0-based), best_x (n,) of +-1.0, G_used (K, r))"""
+        K = int(K)
+        pg = None
+        if G is not None:
+            G, pg = _f64(G)
+            assert G.size == K * self.r, (G.shape, K, self.r)
+        G_used = np.empty((K, self.r), np.float64)
+        obj, tot, x = np.empty(K), np.empty(K), np.empty(self.n)
+        best = C.c_int64()
+        self._check(self.lib.sdplrp_round_hyperplane(self._h, K, pg, int(seed), G_used.ctypes.data_as(_p_f64), obj.ctypes.data_as(_p_f64),
+                                                      tot.ctypes.data_as(_p_f64), C.byref(best), x.ctypes.data_as(_p_f64)))
+        return {"obj": obj, "sum": tot, "best": best.value - 1, "best_x": x, "G_used": G_used}
 
     def solve(self, cfg, r, Rt0=None, lambda0=None, normb=1.0, normC=1.0):
         """sdplrp_solve: the native outer loop -> (Result, best_lambda[m+1])"""

@@ -281,6 +281,22 @@ int32_t comm_gather_rowvec(sdplrp_handle *h, double *v) {
     return SDPLRP_OK;
 }
 
+// the same with row_bytes bytes per row (the packed sign words of the rounding passes)
+int32_t comm_gather_rowbytes(sdplrp_handle *h, void *v, size_t row_bytes) {
+    if (h->world <= 1) return SDPLRP_OK;
+    SectionScope sc(h, SDPLRP_SEC_COMM);
+    ncclComm_t comm = (ncclComm_t)h->nccl;
+    char *p = static_cast<char *>(v);
+    NCCL_TRY(h, ncclGroupStart());
+    for (int q = 0; q < h->world; q++) {
+        const size_t off = (size_t)h->row_starts[(size_t)q] * row_bytes;
+        const size_t len = (size_t)(h->row_starts[(size_t)q + 1] - h->row_starts[(size_t)q]) * row_bytes;
+        if (len > 0) NCCL_TRY(h, ncclBroadcast(p + off, p + off, len, ncclChar, q, comm, h->stream));
+    }
+    NCCL_TRY(h, ncclGroupEnd());
+    return SDPLRP_OK;
+}
+
 // SPMD contract: every rank must have been handed the same problem.  `value` is a 64-bit checksum of this rank's input;
 // the ranks agree iff max == min of both halves (all-reduced as exactly representable doubles).
 int32_t comm_check_same(sdplrp_handle *h, unsigned long long value, const char *what) {

@@ -68,6 +68,16 @@ struct HaloPlan {
     long long sendbuf_len = 0, xc_len = 0;
 };
 
+// hyperplane rounding (rounding.cu): buffers allocated on first use, freed with the problem
+struct RoundingState {
+    unsigned long long *words = nullptr;  // n: one bit per candidate of the current batch, internal vertex order
+    double *x = nullptr;                  // n: the expanded +-1 vector of the best candidate
+    int *chunk_row = nullptr;             // nchunks: first row of every chunk of the evaluation pass
+    long long e_lo = 0, e_hi = 0, nchunks = 0;  // owned nonzeros [e_lo, e_hi) of the full pattern
+    double *G = nullptr, *sums = nullptr; // K x r hyperplanes; 2K + 1 sums (set bits, eval sums, sum of C)
+    long long G_len = 0, sums_len = 0;
+};
+
 struct LowRank {
     i64 gid;     // 0-based global slot
     i64 s;
@@ -246,6 +256,7 @@ struct sdplrp_handle {
     i64 lz_ab_len = 0;
     double *lz_basis = nullptr;
     i64 lz_basis_len = 0;
+    RoundingState rnd;
 };
 
 #define CUDA_TRY(h, call)                                                                      \
@@ -363,6 +374,7 @@ int32_t pre_export(sdplrp_handle *h, int64_t *triu_colptr, int64_t *triu_rowval,
                    int64_t *nzind, double *one, double *two, int64_t *full_colptr, int64_t *full_rowval,
                    int64_t *mapped);
 void pre_free(sdplrp_handle *h);
+void round_free(sdplrp_handle *h);   // rounding buffers (rounding.cu)
 
 // A passes (aop.cu)
 int32_t aop_uu(sdplrp_handle *h, const double *U, double *out_dev);                    // out = A(UU')
@@ -436,6 +448,7 @@ int32_t comm_require_full(sdplrp_handle *h, int mat_id);
 int32_t comm_gather_rows(sdplrp_handle *h, double *p, int mat_id);
 int32_t comm_reduce_mvec(sdplrp_handle *h, double *v1, double *v2);   // shared slots [n_sd, m] only
 int32_t comm_gather_rowvec(sdplrp_handle *h, double *v);              // every rank's owned rows of an n-vector (internal order) to every rank
+int32_t comm_gather_rowbytes(sdplrp_handle *h, void *v, size_t row_bytes);  // the same for row_bytes bytes per row, byte-exact
 int32_t comm_gather_cvec(sdplrp_handle *h, double *v);                // make every per-row-constraint slot current on every rank
 int32_t comm_reduce_scalars(sdplrp_handle *h, int slot, int count);
 int32_t comm_check_same(sdplrp_handle *h, unsigned long long value, const char *what);  // error unless all ranks pass the same value

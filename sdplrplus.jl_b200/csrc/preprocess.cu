@@ -699,6 +699,7 @@ int32_t halo_build(sdplrp_handle *h) {
 void pre_free(sdplrp_handle *h) {
     gather_plan_free(h->full_plan);
     halo_free(h);
+    round_free(h);
     tile_free(h->full_long); tile_free(h->dyn_long);
     dev_free(&h->tile_scratch); h->tile_scratch_len = 0;
     dev_free(&h->row_mid); h->row_mid_cols = -1;

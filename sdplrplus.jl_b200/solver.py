@@ -244,6 +244,10 @@ class B200Engine:
         """k passes of the inner loop body driven inside the library (sdplrp_iterate)."""
         return self.h.iterate(k, alpha_max, use_armijo, update_history)
 
+    def round_hyperplane(self, K, G=None, seed=0):
+        """K hyperplane roundings of the current R on the device (sdplrp_round_hyperplane); see _lib.Handle.round_hyperplane."""
+        return self.h.round_hyperplane(K, G, seed)
+
     def close(self):
         self.h.close()
 
@@ -506,6 +510,20 @@ def _sdplr_native(data, engine, config: BurerMonteiroConfig, r, rng):
         "rankupd_tol": config.rankupd_tol, "r": int(res.r), "lanczos_steps": int(res.lanczos_steps), "L": res.L,
         "status": int(res.status),
     }
+
+
+def hyperplane_rounding(ans, trials=64, seed=0):
+    """Goemans-Williamson rounding of a solve: `trials` random hyperplanes through the factor R that `sdplr` left on the
+    GPU, each cut evaluated on the device.  `ans` is the dict `sdplr` returns.  Returns {"x": the best +-1 vector (input
+    vertex order), "obj": its objective <C, xx'>, "objs": every candidate's objective, "sums": every candidate's sum(x),
+    "trial": the 0-based index of the best candidate}.  Only the objective and the imbalance are evaluated: constraints
+    that a +-1 vector does not satisfy by construction are not checked."""
+    engine = ans["engine"]
+    if not hasattr(engine, "round_hyperplane"):
+        raise TypeError("hyperplane_rounding needs the GPU engine (the rounding passes run inside libsdplrp_b200.so)")
+    out = engine.round_hyperplane(int(trials), None, seed)
+    k = out["best"]
+    return {"x": out["best_x"], "obj": float(out["obj"][k]), "objs": out["obj"], "sums": out["sum"], "trial": k}
 
 
 def _print_row(config, T, localiter, it, L, obj, sigma, gtol, ptol, gn, pn, gap, dual):
