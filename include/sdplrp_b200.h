@@ -286,6 +286,29 @@ int32_t sdplrp_dense_symeig(const double *A, int64_t k, double *ev, double *Q);
  * SDPLRP_ERR_ARG for K < 1, NULL obj / best, and when C has a low-rank part (or no sparse part). */
 int32_t sdplrp_round_hyperplane(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, double *G_out,
                                 double *obj, double *sum, int64_t *best, double *best_x);
+/* Hyperplane rounding followed by parallel one-flip descent on every candidate.  The start vectors x_k^0 are those of
+ * sdplrp_round_hyperplane (same G / seed rule, ties to +1); obj_round[k] (may be NULL) is the objective of x_k^0, bit for
+ * bit the obj[k] of sdplrp_round_hyperplane.  Round t = 0, 1, ... on every candidate k independently: with
+ * h_ik = sum_{j != i} C_ij x_jk, vertex i wants to flip iff x_ik h_ik > 0 (flipping it changes the objective by
+ * -4 x_ik h_ik).  The neighbours of i are the j != i with C_ij != 0.  Priority key(i, t) = mix64(i ^ mix64(0xD1B54A32D192ED03
+ * * (t + 1))) (splitmix64 finalizer, mod 2^64) on the 0-based input vertex index i; j beats i iff key(j, t) > key(i, t), or
+ * the keys are equal and j < i.  Vertex i flips iff it wants to and no neighbour that beats it also wants to: the flipped
+ * vertices are pairwise non-adjacent, their gains add up and the objective falls every round.  A batch of 64 candidates
+ * stops when none of its vertices wants to flip, or after max_rounds rounds.
+ * Outputs: obj[k] = <C, x_k x_k'> of the final vector, sum[k] = sum_i x_{k,i}, flips[k] = single-vertex flips,
+ * rounds[k] = the last (1-based) round that flipped something in candidate k, 0 when x_k^0 is a one-flip local optimum,
+ * -1 when x_k still had a vertex that wanted to flip after max_rounds rounds (not a local optimum).  best (1-based) is the
+ * smallest obj, ties to the lowest k; best_x (reference vertex order) its final vector.  obj_round, sum, flips, rounds,
+ * G_out and best_x may be NULL.  With max_rounds = 0 and rounds NULL this is sdplrp_round_hyperplane.
+ * Candidate k's result does not depend on K or on the other candidates.  Reads R only, like sdplrp_round_hyperplane.
+ * Where the gains are exactly representable (unit-weight MaxCut, +-1-weight cut-norm, integer Laplacians) the results are
+ * bit-identical across vertex orders and GPU counts; with general real weights a gain within rounding of 0 may be decided
+ * differently under a different summation order.
+ * Several GPUs: every rank passes the same K, seed, G and max_rounds and receives the same results.
+ * Errors as sdplrp_round_hyperplane, and SDPLRP_ERR_ARG for max_rounds < 0. */
+int32_t sdplrp_round_local_search(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, int64_t max_rounds,
+                                  double *G_out, double *obj_round, double *obj, double *sum, int64_t *flips,
+                                  int64_t *rounds, int64_t *best, double *best_x);
 
 /* ---- native host driver (SURVEY.md 8f, f1) ------------------------------ */
 /* BurerMonteiroConfig (src/options.jl:1-24); every field is 8 bytes wide so the layout is the same from C, Julia

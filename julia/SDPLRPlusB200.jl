@@ -371,6 +371,27 @@ function round_hyperplane(aux::B200Auxiliary, K::Integer; r::Integer, G=nothing,
     return obj, tot, Int(best[]), x, G_used
 end
 
+"""
+    round_local_search(aux, K; r, G = nothing, seed = 0, max_rounds = 1000)
+        -> (obj_round, obj, sum, flips, rounds, best, best_x, G_used)
+
+The K candidates of `round_hyperplane`, each refined on the device by parallel one-flip descent until no single vertex
+flip lowers <C, xx'> (or `max_rounds` rounds).  `obj_round` are the objectives before the descent, `obj` after,
+`rounds[k]` the last round that flipped candidate k (-1: stopped by `max_rounds`), `best` (1-based) the smallest `obj`
+and `best_x` its +-1 vector.  Reads R only.
+"""
+function round_local_search(aux::B200Auxiliary, K::Integer; r::Integer, G=nothing, seed=0, max_rounds=1000)
+    Gin = G === nothing ? Ptr{Float64}(C_NULL) : Matrix{Float64}(G)
+    G === nothing || size(Gin) == (r, K) || throw(ArgumentError("G must be r x K"))
+    G_used = zeros(r, K); obj0 = zeros(K); obj = zeros(K); tot = zeros(K); flips = zeros(Int64, K); rounds = zeros(Int64, K)
+    best = Ref{Int64}(0); x = zeros(aux.n)
+    GC.@preserve Gin G_used obj0 obj tot flips rounds x check(aux.h, ccall((:sdplrp_round_local_search, LIB), Int32,
+        (Ptr{Cvoid}, Int64, Ptr{Float64}, UInt64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64},
+         Ptr{Int64}, Ref{Int64}, Ptr{Float64}),
+        aux.h.ptr, K, Gin, UInt64(seed), Int64(max_rounds), G_used, obj0, obj, tot, flips, rounds, best, x))
+    return obj0, obj, tot, flips, rounds, Int(best[]), x, G_used
+end
+
 function apply_kwargs!(config, kwargs)
     for (k, v) in kwargs
         hasfield(BurerMonteiroConfig, Symbol(k)) ? setfield!(config, Symbol(k), v) : @error "Unrecognized keyword argument $k"

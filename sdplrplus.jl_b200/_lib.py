@@ -115,6 +115,8 @@ _SIGNATURES.update({
     "sdplrp_iterate": [_H, C.c_int64, C.c_double, C.c_int32, C.c_int32, _p_f64],
     "sdplrp_fill_uniform": [_H, C.c_int32, C.c_uint64],
     "sdplrp_round_hyperplane": [_H, C.c_int64, _p_f64, C.c_uint64, _p_f64, _p_f64, _p_f64, _p_i64, _p_f64],
+    "sdplrp_round_local_search": [_H, C.c_int64, _p_f64, C.c_uint64, C.c_int64, _p_f64, _p_f64, _p_f64, _p_f64, _p_i64, _p_i64, _p_i64,
+                                  _p_f64],
 })
 
 _SPECIAL = {
@@ -535,6 +537,26 @@ class Handle:
         self._check(self.lib.sdplrp_round_hyperplane(self._h, K, pg, int(seed), G_used.ctypes.data_as(_p_f64), obj.ctypes.data_as(_p_f64),
                                                       tot.ctypes.data_as(_p_f64), C.byref(best), x.ctypes.data_as(_p_f64)))
         return {"obj": obj, "sum": tot, "best": best.value - 1, "best_x": x, "G_used": G_used}
+
+    def round_local_search(self, K, G=None, seed=0, max_rounds=1000):
+        """sdplrp_round_local_search: the K hyperplane roundings of round_hyperplane, each refined by one-flip descent ->
+        dict(obj_round (K,) before the descent, obj (K,), sum (K,), flips (K,), rounds (K,; -1 = stopped by max_rounds),
+        best (0-based), best_x (n,) of +-1.0, G_used (K, r))"""
+        K = int(K)
+        pg = None
+        if G is not None:
+            G, pg = _f64(G)
+            assert G.size == K * self.r, (G.shape, K, self.r)
+        G_used = np.empty((K, self.r), np.float64)
+        obj0, obj, tot, x = np.empty(K), np.empty(K), np.empty(K), np.empty(self.n)
+        flips, rounds = np.empty(K, np.int64), np.empty(K, np.int64)
+        best = C.c_int64()
+        self._check(self.lib.sdplrp_round_local_search(
+            self._h, K, pg, int(seed), int(max_rounds), G_used.ctypes.data_as(_p_f64), obj0.ctypes.data_as(_p_f64),
+            obj.ctypes.data_as(_p_f64), tot.ctypes.data_as(_p_f64), flips.ctypes.data_as(_p_i64), rounds.ctypes.data_as(_p_i64),
+            C.byref(best), x.ctypes.data_as(_p_f64)))
+        return {"obj_round": obj0, "obj": obj, "sum": tot, "flips": flips, "rounds": rounds, "best": best.value - 1, "best_x": x,
+                "G_used": G_used}
 
     def solve(self, cfg, r, Rt0=None, lambda0=None, normb=1.0, normC=1.0):
         """sdplrp_solve: the native outer loop -> (Result, best_lambda[m+1])"""

@@ -74,8 +74,18 @@ struct RoundingState {
     double *x = nullptr;                  // n: the expanded +-1 vector of the best candidate
     int *chunk_row = nullptr;             // nchunks: first row of every chunk of the evaluation pass
     long long e_lo = 0, e_hi = 0, nchunks = 0;  // owned nonzeros [e_lo, e_hi) of the full pattern
-    double *G = nullptr, *sums = nullptr; // K x r hyperplanes; 2K + 1 sums (set bits, eval sums, sum of C)
+    double *G = nullptr, *sums = nullptr; // K x r hyperplanes; per batch 4 x 64 sums (set bits, eval sums, first eval sums,
+                                          // flips), then sum of C and 64 want counts of a local-search round
     long long G_len = 0, sums_len = 0;
+    // one-flip local search (first use)
+    unsigned long long *want = nullptr, *flip = nullptr;  // n: want / flip word of every vertex in the current round
+    unsigned long long *best_words = nullptr;             // n: final words of the batch that holds the best candidate so far
+    unsigned char *dirty = nullptr;                       // n: the row's want word must be recomputed
+    int *long_rows = nullptr, *long_sptr = nullptr;       // rows of the full pattern with more than kLsLong nonzeros (ascending),
+                                                          // and the first segment of each (+1)
+    int *seg_row = nullptr, *seg_start = nullptr;         // n_seg: row and first nonzero of every segment
+    double *seg_part = nullptr;                           // n_seg x 64 want sums of a segment
+    long long n_seg = 0, l_lo = 0, l_hi = 0, s_lo = 0, s_hi = 0;  // the owned long rows [l_lo, l_hi) and their segments [s_lo, s_hi)
 };
 
 struct LowRank {

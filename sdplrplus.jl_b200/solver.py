@@ -248,6 +248,11 @@ class B200Engine:
         """K hyperplane roundings of the current R on the device (sdplrp_round_hyperplane); see _lib.Handle.round_hyperplane."""
         return self.h.round_hyperplane(K, G, seed)
 
+    def round_local_search(self, K, G=None, seed=0, max_rounds=1000):
+        """K hyperplane roundings refined by one-flip descent on the device (sdplrp_round_local_search); see
+        _lib.Handle.round_local_search."""
+        return self.h.round_local_search(K, G, seed, max_rounds)
+
     def close(self):
         self.h.close()
 
@@ -512,18 +517,27 @@ def _sdplr_native(data, engine, config: BurerMonteiroConfig, r, rng):
     }
 
 
-def hyperplane_rounding(ans, trials=64, seed=0):
+def hyperplane_rounding(ans, trials=64, seed=0, local_search_rounds=0):
     """Goemans-Williamson rounding of a solve: `trials` random hyperplanes through the factor R that `sdplr` left on the
     GPU, each cut evaluated on the device.  `ans` is the dict `sdplr` returns.  Returns {"x": the best +-1 vector (input
     vertex order), "obj": its objective <C, xx'>, "objs": every candidate's objective, "sums": every candidate's sum(x),
     "trial": the 0-based index of the best candidate}.  Only the objective and the imbalance are evaluated: constraints
-    that a +-1 vector does not satisfy by construction are not checked."""
+    that a +-1 vector does not satisfy by construction are not checked.
+    local_search_rounds > 0: every candidate is then refined by at most that many rounds of parallel one-flip descent
+    on the device (sdplrp_round_local_search), and "x", "obj", "objs", "sums" describe the refined candidates; the result
+    also has "objs_rounded" (before the descent), "flips" and "rounds" (per candidate; -1 = stopped by the round limit)."""
     engine = ans["engine"]
     if not hasattr(engine, "round_hyperplane"):
         raise TypeError("hyperplane_rounding needs the GPU engine (the rounding passes run inside libsdplrp_b200.so)")
-    out = engine.round_hyperplane(int(trials), None, seed)
+    if local_search_rounds > 0:
+        out = engine.round_local_search(int(trials), None, seed, int(local_search_rounds))
+    else:
+        out = engine.round_hyperplane(int(trials), None, seed)
     k = out["best"]
-    return {"x": out["best_x"], "obj": float(out["obj"][k]), "objs": out["obj"], "sums": out["sum"], "trial": k}
+    res = {"x": out["best_x"], "obj": float(out["obj"][k]), "objs": out["obj"], "sums": out["sum"], "trial": k}
+    if local_search_rounds > 0:
+        res.update(objs_rounded=out["obj_round"], flips=out["flips"], rounds=out["rounds"])
+    return res
 
 
 def _print_row(config, T, localiter, it, L, obj, sigma, gtol, ptol, gn, pn, gap, dual):
