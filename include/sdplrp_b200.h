@@ -175,7 +175,14 @@ int32_t sdplrp_set_problem(sdplrp_handle *h, const double *b, const uint8_t *is_
 
 /* ---- state: SolverVars / LBFGSHistory --------------------------------- */
 /* (re)allocates R,G,D and the 2*numlbfgsvecs history for rank r and clears the
- * history (lbfgs_init, src/lbfgs.jl:35-47; rank_update!, src/coreop.jl:518-526) */
+ * history (lbfgs_init, src/lbfgs.jl:35-47; rank_update!, src/coreop.jl:518-526).
+ * Supported ranks: 1 <= r <= SDPLRP_MAX_RANK (256), and r <= SDPLRP_MAX_ODD_RANK (128)
+ * when r is odd -- the sparse row kernels hold at most 4 x 32 lanes of 2 (even r) or
+ * 1 (odd r) columns per row.  Any other r returns SDPLRP_ERR_ARG before anything is
+ * allocated or launched; the previous rank and state stay valid.  sdplrp_solve's rank
+ * update clamps min(barvinok_pataki, 2r) to this range (an odd r > 128 steps down by 1). */
+#define SDPLRP_MAX_RANK 256
+#define SDPLRP_MAX_ODD_RANK 128
 int32_t sdplrp_set_rank(sdplrp_handle *h, int32_t r, int32_t numlbfgsvecs);
 int32_t sdplrp_set_sigma(sdplrp_handle *h, double sigma);
 int32_t sdplrp_get_sigma(sdplrp_handle *h, double *sigma);

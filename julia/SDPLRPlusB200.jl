@@ -321,9 +321,15 @@ function dual_obj(data, var::SolverVars{Ti,Float64,DevMat}, aux::B200Auxiliary, 
     return dual[], lam[]
 end
 
+# min(bp, 2r) clamped to the ranks sdplrp_set_rank accepts (r <= 256, odd r <= 128): the rule of sdplrp_solve and solver.py
+function rank_after_update(bp::Integer, r::Integer)
+    t = min(bp, 2r, 256)
+    return (isodd(t) && t > 128) ? t - 1 : t
+end
+
 # src/coreop.jl:518-526  rank_update!(data, var, config): a fresh point of the new rank on the device
 function rank_update!(data, var::SolverVars{Ti,Float64,DevMat}, config::BurerMonteiroConfig{Ti,Float64}) where {Ti<:Integer}
-    newr = min(barvinok_pataki(data), var.r[] * 2)
+    newr = rank_after_update(barvinok_pataki(data), var.r[])
     set_rank!(data, newr)
     h = var.Rt.h
     return device_vars(data, B200Auxiliary(h, size(var.Rt, 2), length(var.λ)), newr, config)

@@ -355,6 +355,11 @@ int32_t sdplrp_set_rank(sdplrp_handle *h, int32_t r, int32_t numlbfgsvecs) {
     REQUIRE_H(h);
     REQUIRE_PRE(h);
     if (r < 1 || numlbfgsvecs < 0 || numlbfgsvecs > kMaxHist) return fail(h, SDPLRP_ERR_ARG, "set_rank: bad rank / history length");
+    // checked before anything is freed or launched: the sparse row kernels would fail later (r > 128 odd) or the per-row
+    // constraint tile pass would get zero rows per tile (r > 256 odd, r > 512 even)
+    if (!rank_supported(r))
+        return fail(h, SDPLRP_ERR_ARG, "set_rank: r = " + std::to_string(r) + " is not supported (r <= " + std::to_string(SDPLRP_MAX_RANK) +
+                                           ", and r <= " + std::to_string(SDPLRP_MAX_ODD_RANK) + " when r is odd)");
     CUDA_TRY(h, cudaSetDevice(h->device));
     const i64 N = mat_capacity(h, r);
     // same rank, history length and capacity as the current state (a new start point for the same problem, the e2e path of

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <algorithm>
 #include <string>
 #include <vector>
 #include "../../include/sdplrp_b200.h"
@@ -20,6 +21,19 @@ constexpr int kLongMatThreshold = 64;   // matrices with more triu entries go to
 constexpr int kChunkEntries = 2048;     // entries per chunk (one CTA) of a long matrix
 constexpr int kRowGroupMax = 64;        // rows with <= this many nonzeros: one sub-warp lane group per row
 constexpr int kRowWarpMax = 512;        // rows with <= this many: one warp per row; longer: chunks of this size, one warp each
+
+// the ranks every kernel handles (include/sdplrp_b200.h, sdplrp_set_rank): at most 4 units of 32 lanes per row in the sparse
+// row kernels (gradient.cu, launch_csr), each lane holding 2 columns for even r and 1 for odd r
+static inline bool rank_supported(long long r) {
+    return r >= 1 && r <= SDPLRP_MAX_RANK && (r % 2 == 0 || r <= SDPLRP_MAX_ODD_RANK);
+}
+// rank_update! (src/coreop.jl:518-526) r <- min(bp, 2r), clamped to the largest supported rank at or below it
+// (solver.py rank_after_update is the same rule)
+static inline long long rank_after_update(long long bp, long long r) {
+    long long t = std::min(std::min(bp, 2 * r), (long long)SDPLRP_MAX_RANK);
+    if (t % 2 == 1 && t > SDPLRP_MAX_ODD_RANK) t -= 1;
+    return t;
+}
 
 // rows of a CSR pattern binned by length (compacted lists, natural order inside a bin);
 // list[c] == nullptr with cnt[c] == n means "all rows" (identity, keeps streaming access)

@@ -248,6 +248,7 @@ int32_t sdplrp_solve(sdplrp_handle *h, const sdplrp_config *cfgp, int64_t r0, co
     if (!h) return SDPLRP_ERR_ARG;
     if (!h->preprocessed) return fail(h, SDPLRP_ERR_STATE, "solve: sdplrp_preprocess / sdplrp_set_problem first");
     if (!cfgp || !res || r0 < 1) return fail(h, SDPLRP_ERR_ARG, "solve: bad argument");
+    if (!rank_supported(r0)) return fail(h, SDPLRP_ERR_ARG, "solve: initial rank " + std::to_string(r0) + " is not supported (see sdplrp_set_rank)");
     const sdplrp_config &cfg = *cfgp;
     Driver drv{h, cfg};
     const i64 n = h->n, m = h->m;
@@ -368,9 +369,10 @@ int32_t sdplrp_solve(sdplrp_handle *h, const sdplrp_config *cfgp, int64_t r0, co
         }
 
         if (rank_double) {
-            // rank_update! (src/coreop.jl:518-526): brand-new random variables, r <- min(barvinok_pataki, 2r), sigma <- sigma_0
+            // rank_update! (src/coreop.jl:518-526): brand-new random variables, r <- min(barvinok_pataki, 2r), sigma <- sigma_0;
+            // r is clamped to the supported ranks (<= 256, odd <= 128), and may stay the same
             const i64 bp = std::min<i64>(n, (i64)floor(sqrt(2.0 * (double)m) + 1.0));
-            r = std::min<i64>(bp, 2 * r);
+            r = rank_after_update(bp, r);
             SDP_CHECK(init_point(r, nullptr, nullptr));
             sigma = cfg.sigma_0;
             cur_ptol = 1.0 / pow(sigma, 0.1);

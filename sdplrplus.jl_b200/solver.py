@@ -90,6 +90,22 @@ def barvinok_pataki(n, m):
     return min(n, int(math.floor(math.sqrt(2 * m) + 1)))
 
 
+MAX_RANK = 256       # SDPLRP_MAX_RANK: the largest rank sdplrp_set_rank accepts
+MAX_ODD_RANK = 128   # SDPLRP_MAX_ODD_RANK: the largest odd rank
+
+
+def rank_supported(r):
+    """The ranks the GPU kernels handle (include/sdplrp_b200.h, sdplrp_set_rank)."""
+    return 1 <= r <= MAX_RANK and (r % 2 == 0 or r <= MAX_ODD_RANK)
+
+
+def rank_after_update(bp, r):
+    """rank_update! (src/coreop.jl:518-526): r <- min(bp, 2r), clamped to the largest supported rank at or below it (an odd
+    rank above 128 steps down by 1).  The same rule as rank_after_update in csrc/common.cuh (the native driver)."""
+    t = min(bp, 2 * r, MAX_RANK)
+    return t - 1 if t % 2 == 1 and t > MAX_ODD_RANK else t
+
+
 def pick_alpha(bq, alpha_max=1.0):
     """Root selection of linesearch! (src/linesearch.jl:58-112): minimise the
     quartic over the real roots of its derivative in [0, alpha_max] and alpha_max.
@@ -439,8 +455,8 @@ def _sdplr(data, engine, config: BurerMonteiroConfig, stats: SolverStats, r, rng
             cur_gtol = 1.0 / sigma
 
         if rank_double:
-            # rank_update! (src/coreop.jl:518-526): brand-new variables, r <- min(BP, 2r), sigma <- sigma_0
-            r = min(barvinok_pataki(n, m), 2 * r)
+            # rank_update! (src/coreop.jl:518-526): brand-new variables, r <- min(BP, 2r) clamped to the supported ranks, sigma <- sigma_0
+            r = rank_after_update(barvinok_pataki(n, m), r)
             Rt_new, lam_new = _init_point(data, r, config, rng)
             engine.init_vars(r, Rt_new, lam_new, config.sigma_0, config.numlbfgsvecs)
             sigma = config.sigma_0

@@ -99,6 +99,26 @@ def test_misc(sp):
     assert sp.frobenius_norm(sps.csc_matrix(np.array([[3.0, 0], [0, 4.0]]))) == 5.0
 
 
+def test_rank_update_clamp(sp):
+    """rank_after_update (the rank update of both drivers): always a supported rank, never above min(bp, 2r), and the
+    largest supported rank at or below it; the limits are the ones include/sdplrp_b200.h states"""
+    import os
+    import re
+    S = sp.solver
+    hdr = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "sdplrp_b200.h")).read()
+    assert int(re.search(r"#define SDPLRP_MAX_RANK (\d+)", hdr).group(1)) == S.MAX_RANK == 256
+    assert int(re.search(r"#define SDPLRP_MAX_ODD_RANK (\d+)", hdr).group(1)) == S.MAX_ODD_RANK == 128
+    supported = [t for t in range(1, 600) if S.rank_supported(t)]
+    assert supported == list(range(1, 129)) + list(range(130, 257, 2))
+    for bp in (1, 2, 3, 41, 127, 128, 129, 130, 200, 255, 256, 257, 258, 283, 1000, 10 ** 6):
+        for r in range(1, 301):
+            want = min(bp, 2 * r)
+            t = S.rank_after_update(bp, r)
+            assert S.rank_supported(t) and t <= want, (bp, r, t)
+            assert t == max(u for u in supported if u <= want), (bp, r, t)
+    assert S.rank_after_update(283, 160) == 256 and S.rank_after_update(201, 128) == 200 and S.rank_after_update(41, 40) == 41
+
+
 def _scaled_quartics(count, seed):
     """quartic coefficient sets over seven orders of magnitude, including the degenerate shapes of the line search"""
     rng = np.random.default_rng(seed)
