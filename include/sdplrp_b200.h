@@ -103,6 +103,8 @@ void *sdplrp_stream(sdplrp_handle *h);
  *                 warp each; set BEFORE sdplrp_preprocess
  *   "spmm_unroll" nonzeros per block of the short-row kernels: 8 (default) or 4
  *   "spmm_g0"     1 = lane groups of exactly r/2 lanes per short row (default: 6 rows per warp at r = 10), 0 = next power of two
+ *   "obj_value_free" 1 = when every off-diagonal value of C is the same +-2^k (unweighted MaxCut: 0.25) the gather pass
+ *                 CD = C*D reads only C's pattern and scales each row once (default; same bits), 0 = it always reads C's values
  *   "rowc_kernel" pass over the per-row (single-diagonal-entry) constraints: 1 = barrier-free warp kernel, 32/(r/2) whole rows per
  *                 warp step (default on one GPU; rows of at most 32 pieces), 0 = shared-memory tile kernel (always on several GPUs).  Same bits either way
  *   "tail_ctas"   CTAs per SM of the fused step + gradient pass (1..8; 0 = auto, the default: 6 on one GPU, 4 on several.  Measured on C5, one GPU:
@@ -161,6 +163,10 @@ typedef struct {
 } sdplrp_block;
 int32_t sdplrp_preprocess_blocks(sdplrp_handle *h, int64_t n, int64_t m, int64_t nblocks, const sdplrp_block *blocks);
 int32_t sdplrp_pattern_sizes(sdplrp_handle *h, int64_t *nnzT, int64_t *nnzF, int64_t *Ec);
+/* the weight v that the one-sweep row kernels of the gather pass CD = C*D factor out of C ("obj_value_free"), 0 when they
+ * read C's values.  The asynchronous tile pipeline ("gather_mode"), the two-phase pass ("spmm_phases") and the halo pass of
+ * several GPUs always read the values */
+int32_t sdplrp_value_free_weight(sdplrp_handle *h, double *v);
 /* 1-based, exactly the seven outputs of preprocess_sparsecons (SURVEY Appendix B) */
 int32_t sdplrp_pattern_export(sdplrp_handle *h, int64_t *triu_colptr, int64_t *triu_rowval, int64_t *matptr,
                               int64_t *nzind, double *nzval_one, double *nzval_two, int64_t *full_colptr,

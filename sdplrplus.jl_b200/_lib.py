@@ -47,6 +47,7 @@ _SIGNATURES = {
     "sdplrp_preprocess_blocks": [_H, C.c_int64, C.c_int64, C.c_int64, C.POINTER(Block)],
     "sdplrp_halo_stats": [_H, _p_i64],
     "sdplrp_pattern_sizes": [_H, _p_i64, _p_i64, _p_i64],
+    "sdplrp_value_free_weight": [_H, _p_f64],
     "sdplrp_pattern_export": [_H, _p_i64, _p_i64, _p_i64, _p_i64, _p_f64, _p_f64, _p_i64, _p_i64, _p_i64],
     "sdplrp_add_symlowrank": [_H, C.c_int64, C.c_int64, _p_f64, _p_f64],
     "sdplrp_set_problem": [_H, _p_f64, _p_u8],
@@ -287,6 +288,12 @@ class Handle:
         a, b, c = C.c_int64(), C.c_int64(), C.c_int64()
         self._check(self.lib.sdplrp_pattern_sizes(self._h, C.byref(a), C.byref(b), C.byref(c)))
         return a.value, b.value, c.value
+
+    def value_free_weight(self):
+        """The weight v the gather pass CD = C*D factors out of C (option "obj_value_free"); 0.0 when it reads C's values."""
+        v = C.c_double()
+        self._check(self.lib.sdplrp_value_free_weight(self._h, C.byref(v)))
+        return v.value
 
     def pattern_export(self):
         nnzT, nnzF, Ec = self.pattern_sizes()

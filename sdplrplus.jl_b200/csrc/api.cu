@@ -294,6 +294,14 @@ int32_t sdplrp_halo_stats(sdplrp_handle *h, int64_t out[7]) {
     return SDPLRP_OK;
 }
 
+int32_t sdplrp_value_free_weight(sdplrp_handle *h, double *v) {
+    REQUIRE_H(h);
+    REQUIRE_PRE(h);
+    if (!v) return fail(h, SDPLRP_ERR_ARG, "value_free_weight: null pointer");
+    *v = obj_value_free(h) ? h->vf_val : 0.0;
+    return SDPLRP_OK;
+}
+
 int32_t sdplrp_pattern_sizes(sdplrp_handle *h, int64_t *nnzT, int64_t *nnzF, int64_t *Ec) {
     REQUIRE_H(h);
     REQUIRE_PRE(h);
@@ -398,6 +406,7 @@ int32_t sdplrp_set_option(sdplrp_handle *h, const char *key, double value) {
     if (k == "row_group_max") { h->row_group_max = std::max(1, std::min((int)value, kRowWarpMax)); return SDPLRP_OK; }   // before preprocess
     if (k == "spmm_unroll") { h->spmm_unroll = (int)value; return SDPLRP_OK; }
     if (k == "spmm_g0") { h->spmm_g0 = (int)value; return SDPLRP_OK; }
+    if (k == "obj_value_free") { h->obj_value_free = value != 0 ? 1 : 0; return SDPLRP_OK; }
     if (k == "rowc_kernel") { h->rowc_kernel = value > 0 ? 1 : 0; return SDPLRP_OK; }
     if (k == "tail_ctas") { h->tail_ctas = std::max(0, std::min((int)value, 8)); return SDPLRP_OK; }
     if (k == "halo") { h->halo_mode = value < 0.5 ? 0 : (value < 1.5 ? 1 : (value < 2.5 ? 2 : 3)); return SDPLRP_OK; }

@@ -215,6 +215,11 @@ struct sdplrp_handle {
     int *dyn_pos_a = nullptr, *dyn_pos_b = nullptr;  // n_dyn: the (row,col) and (col,row) slots of the full pattern
     // objective-split hot path: static objective values on the full pattern, dynamic pattern as CSR
     double *Cfull = nullptr;       // nnzF: C's value at every full-pattern slot (0 where C has no entry)
+    // value-free gather pass (gradient.cu, grad_obj_spmm): every off-diagonal Cfull value is the same v = +-2^k (unweighted
+    // MaxCut: 0.25), so C*X = v * (pattern*X with C_ii / v on the diagonal), bit for bit; set by pre_build
+    double vf_val = 0.0;           // v, 0 = C is not of that form
+    double *vf_diag = nullptr;     // n: C_ii / v (0 where the pattern has no diagonal entry)
+    int obj_value_free = 1;        // sdplrp_set_option "obj_value_free": 0 = always read Cfull (A/B, tests)
     double *dynS = nullptr;        // n_dyn: constraint part of S at the dynamic slots (per iteration)
     i64 n_dynF = 0;                // dynamic slots of the full pattern
     int *dynrow_ptr = nullptr;     // n+1
@@ -415,6 +420,7 @@ int32_t grad_assemble_S(sdplrp_handle *h);                      // At_preprocess
 int32_t grad_spmm(sdplrp_handle *h, const double *X, double *Y, double scale, bool want_norm);  // Y = scale*X*S (+low rank)
 int32_t grad_spmm_sparse(sdplrp_handle *h, const double *X, double *Y, double scale);           // Y = scale*X*S, sparse part only
 int32_t grad_obj_spmm(sdplrp_handle *h, const double *X, double *Y, const double *Z, double *sums6);  // Y = C*X, sums <X,Y>, <X,Z>
+inline bool obj_value_free(const sdplrp_handle *h) { return h->obj_value_free && h->vf_val != 0.0; }  // grad_obj_spmm skips Cfull
 int32_t grad_obj_slots(sdplrp_handle *h, const double *sums6, double *a_rd_m, double *a_dd_m);
 int32_t grad_hot(sdplrp_handle *h);                             // G = 2*(y_obj*CR + S_dyn*R + low rank), ||G||^2
 int32_t grad_step_fused(sdplrp_handle *h, double alpha);        // step + y + gradient + both norms in one row pass

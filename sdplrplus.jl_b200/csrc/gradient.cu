@@ -211,9 +211,13 @@ struct RowArgs {
     const int *chunk_start, *chunk_end, *chunk_row;
     const int *long_rows, *long_cptr;
     double *scratch;
+    // VF (value-free rows, uniform off-diagonal C = vf_scale = +-2^k): the nonzeros contribute X_j unscaled, the diagonal
+    // contributes (C_ii / vf_scale) * X_i, and the row total is scaled once -- the same bits as the valued sum
+    const double *vf_diag;
+    double vf_scale;
 };
 
-template <int VEC, int MAXU, int EPI>
+template <int VEC, int MAXU, int EPI, bool VF = false>
 __device__ __forceinline__ void row_epilogue(const RowArgs &a, i64 i, Acc<VEC> (&acc)[MAXU], int lg, int nv, double &s0, double &s1,
                                              int G) {
 #pragma unroll
@@ -221,6 +225,7 @@ __device__ __forceinline__ void row_epilogue(const RowArgs &a, i64 i, Acc<VEC> (
         const int c = lg + u * G;
         if (c < nv) {
             const size_t off = (size_t)i * a.r + c * VEC;
+            if (VF) acc[u].scale(a.vf_scale);   // exact: a power of two
             if (EPI == 0) {
                 acc[u].scale(a.scale);
             } else if (EPI == 3) {
@@ -284,8 +289,10 @@ __device__ __forceinline__ void finish_sums(const RowArgs &a, double s0, double 
 // class 0: one group of G0 lanes per row (G0 = pieces per row when that fits a warp: 6 rows per warp at r = 10);
 // the row's nonzeros are taken NB at a time, fully predicated, so a row of <= NB nonzeros costs one round trip
 // ptr -> idx/val -> gathers with NB independent 128-bit gathers in flight per lane
-template <int VEC, int MAXU, bool IND, int EPI, int NB>
-__global__ void LB_GROUP k_rows_group(RowArgs a) {
+// VF: the rows carry no values (RowArgs::vf_diag): every nonzero weighs 1 except the diagonal
+// (VF, one unit per row: at most 64 registers, 4 CTAs per SM as the valued kernel; ptxas would otherwise take 66 and drop to 3)
+template <int VEC, int MAXU, bool IND, int EPI, int NB, bool VF>
+__global__ void __launch_bounds__(TPB, VF && MAXU == 1 ? 4 : SDPLRP_LB_GROUP) k_rows_group(RowArgs a) {
     const int nv = a.r / VEC;
     const int G = a.G0;
     const int gpb = TPB / G;                       // groups per CTA (lanes beyond gpb*G idle)
@@ -301,6 +308,7 @@ __global__ void LB_GROUP k_rows_group(RowArgs a) {
         const i64 i = a.rows ? a.rows[q] : q;
         if (i < a.own_lo || i >= a.own_hi) continue;
         const int beg = a.beg_arr ? a.beg_arr[i] : a.ptr[i], end = a.end_arr ? a.end_arr[i] : a.ptr[i + 1];
+        const double dii = VF ? a.vf_diag[i] : 0.0;
         Acc<VEC> acc[MAXU];
 #pragma unroll
         for (int u = 0; u < MAXU; u++) acc[u].zero();
@@ -311,19 +319,31 @@ __global__ void LB_GROUP k_rows_group(RowArgs a) {
             for (int j = 0; j < NB; j++) {
                 const bool ok = k0 + j < end;
                 cc[j] = ok ? ldg_i32_hint(a.idx + k0 + j, p_str) : 0;
-                vv[j] = ok ? (IND ? __ldg(a.val + ldg_i32_hint(a.src + k0 + j, p_str)) : ldg_f64_hint(a.val + k0 + j, p_str)) : 0.0;
+                if (VF) vv[j] = ok ? (cc[j] == (int)i ? dii : 1.0) : 0.0;
+                else vv[j] = ok ? (IND ? __ldg(a.val + ldg_i32_hint(a.src + k0 + j, p_str)) : ldg_f64_hint(a.val + k0 + j, p_str)) : 0.0;
             }
 #pragma unroll
             for (int u = 0; u < MAXU; u++) {
                 const int c = lg + u * G;
                 if (c < nv) {
+                    if (VF) {   // every gather of the block issued before the first use (vv = 0 past the row's end)
+                        Acc<VEC> x[NB];
 #pragma unroll
-                    for (int j = 0; j < NB; j++)
-                        if (k0 + j < end) acc[u].fma_hint(vv[j], a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                        for (int j = 0; j < NB; j++) {
+                            x[j].zero();
+                            if (k0 + j < end) x[j].ld_hint(a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                        }
+#pragma unroll
+                        for (int j = 0; j < NB; j++) acc[u].fma_reg(vv[j], x[j]);
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < NB; j++)
+                            if (k0 + j < end) acc[u].fma_hint(vv[j], a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                    }
                 }
             }
         }
-        row_epilogue<VEC, MAXU, EPI>(a, i, acc, lg, nv, s0, s1, G);
+        row_epilogue<VEC, MAXU, EPI, VF>(a, i, acc, lg, nv, s0, s1, G);
     }
     finish_sums<EPI>(a, s0, s1);
 }
@@ -332,7 +352,7 @@ __global__ void LB_GROUP k_rows_group(RowArgs a) {
 // CHUNK: the work items are the kRowWarpMax-nonzero chunks of the long rows (class 2) and the warp leaves its partial
 // sums in a.scratch (combined per row, in chunk order, by k_rows_combine) -- a hub row of 30 k nonzeros is spread over
 // 60 warps instead of serialising one CTA, which is what lets the pass scale when the rows are divided among GPUs.
-template <int VEC, int MAXU, bool IND, int EPI, bool CHUNK>
+template <int VEC, int MAXU, bool IND, int EPI, bool CHUNK, bool VF>
 __global__ void LB_WARP k_rows_warp(RowArgs a) {
     const int nv = a.r / VEC;
     const int lane = threadIdx.x & 31;
@@ -351,6 +371,7 @@ __global__ void LB_WARP k_rows_warp(RowArgs a) {
         if (i < a.own_lo || i >= a.own_hi) continue;
         const int beg = CHUNK ? a.chunk_start[q] : (a.beg_arr ? a.beg_arr[i] : a.ptr[i]);
         const int end = CHUNK ? a.chunk_end[q] : (a.end_arr ? a.end_arr[i] : a.ptr[i + 1]);
+        const double dii = VF ? a.vf_diag[i] : 0.0;
         Acc<VEC> acc[MAXU];
 #pragma unroll
         for (int u = 0; u < MAXU; u++) acc[u].zero();
@@ -361,15 +382,27 @@ __global__ void LB_WARP k_rows_warp(RowArgs a) {
             for (int j = 0; j < 4; j++) {
                 const bool ok = k0 + j < end;
                 cc[j] = ok ? ldg_i32_hint(a.idx + k0 + j, p_str) : 0;
-                vv[j] = ok ? (IND ? __ldg(a.val + ldg_i32_hint(a.src + k0 + j, p_str)) : ldg_f64_hint(a.val + k0 + j, p_str)) : 0.0;
+                if (VF) vv[j] = ok ? (cc[j] == (int)i ? dii : 1.0) : 0.0;
+                else vv[j] = ok ? (IND ? __ldg(a.val + ldg_i32_hint(a.src + k0 + j, p_str)) : ldg_f64_hint(a.val + k0 + j, p_str)) : 0.0;
             }
 #pragma unroll
             for (int u = 0; u < MAXU; u++) {
                 const int c = lg + u * Gw;
                 if (c < nv) {
+                    if (VF) {   // every gather of the block issued before the first use (vv = 0 past the row's end)
+                        Acc<VEC> x[4];
 #pragma unroll
-                    for (int j = 0; j < 4; j++)
-                        if (k0 + j < end) acc[u].fma_hint(vv[j], a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                        for (int j = 0; j < 4; j++) {
+                            x[j].zero();
+                            if (k0 + j < end) x[j].ld_hint(a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                        }
+#pragma unroll
+                        for (int j = 0; j < 4; j++) acc[u].fma_reg(vv[j], x[j]);
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 4; j++)
+                            if (k0 + j < end) acc[u].fma_hint(vv[j], a.X + (size_t)cc[j] * a.r + c * VEC, cc[j] < a.hot_rows ? p_hot : p_str);
+                    }
                 }
             }
         }
@@ -394,7 +427,7 @@ __global__ void LB_WARP k_rows_warp(RowArgs a) {
                     if (c < nv) acc[u].store(a.scratch + (size_t)q * a.r + c * VEC);
                 }
             } else {
-                row_epilogue<VEC, MAXU, EPI>(a, i, acc, lg, nv, s0, s1, Gw);
+                row_epilogue<VEC, MAXU, EPI, VF>(a, i, acc, lg, nv, s0, s1, Gw);
             }
         }
     }
@@ -402,7 +435,7 @@ __global__ void LB_WARP k_rows_warp(RowArgs a) {
 }
 
 // class 2, second step: per long row the chunk partials are added in chunk order, then the row epilogue
-template <int VEC, int MAXU, int EPI>
+template <int VEC, int MAXU, int EPI, bool VF>
 __global__ void __launch_bounds__(TPB) k_rows_combine(RowArgs a) {
     const int nv = a.r / VEC;
     const int lg = threadIdx.x & (a.G - 1);
@@ -422,7 +455,7 @@ __global__ void __launch_bounds__(TPB) k_rows_combine(RowArgs a) {
                 if (p < nv) acc[u].add_mem(a.scratch + (size_t)c * a.r + p * VEC);
             }
         }
-        row_epilogue<VEC, MAXU, EPI>(a, i, acc, lg, nv, s0, s1, a.G);
+        row_epilogue<VEC, MAXU, EPI, VF>(a, i, acc, lg, nv, s0, s1, a.G);
     }
     finish_sums<EPI>(a, s0, s1);
 }
@@ -633,7 +666,7 @@ static int32_t classes_join(sdplrp_handle *h) {
     return SDPLRP_OK;
 }
 
-template <int VEC, int MAXU, bool IND, int EPI>
+template <int VEC, int MAXU, bool IND, int EPI, bool VF>
 int32_t launch_classes(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const TileLayout &longs, double *sums /* 3 x 2 or null */,
                        bool long_empty = false, int class_mask = 7) {
     const int gpb = TPB / a.G;
@@ -659,14 +692,14 @@ int32_t launch_classes(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const
             continue;
         }
         if (c == 0) {
-            if (h->spmm_unroll >= 8) k_rows_group<VEC, MAXU, IND, EPI, 8><<<grid_for(a.n_rows, gpb0, spmm_cap), TPB, 0, st>>>(a);
-            else k_rows_group<VEC, MAXU, IND, EPI, 4><<<grid_for(a.n_rows, gpb0, spmm_cap), TPB, 0, st>>>(a);
+            if (h->spmm_unroll >= 8) k_rows_group<VEC, MAXU, IND, EPI, 8, VF><<<grid_for(a.n_rows, gpb0, spmm_cap), TPB, 0, st>>>(a);
+            else k_rows_group<VEC, MAXU, IND, EPI, 4, VF><<<grid_for(a.n_rows, gpb0, spmm_cap), TPB, 0, st>>>(a);
         } else if (c == 1) {
-            k_rows_warp<VEC, MAXU, IND, EPI, false><<<grid_for(a.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(a);
+            k_rows_warp<VEC, MAXU, IND, EPI, false, VF><<<grid_for(a.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(a);
         } else if (long_empty) {
             RowArgs b = a;
             b.beg_arr = a.ptr + 1; b.end_arr = a.ptr + 1;
-            k_rows_warp<VEC, MAXU, IND, EPI, false><<<grid_for(b.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(b);
+            k_rows_warp<VEC, MAXU, IND, EPI, false, VF><<<grid_for(b.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(b);
         } else {
             // long rows: one warp per chunk, then the per-row combination with the epilogue
             const i64 need = longs.n_chunks * (i64)a.r;
@@ -679,10 +712,10 @@ int32_t launch_classes(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const
             b.chunk_start = longs.chunk_start; b.chunk_end = longs.chunk_end; b.chunk_row = longs.chunk_row;
             b.long_rows = longs.long_rows; b.long_cptr = longs.long_cptr; b.scratch = h->tile_scratch;
             b.n_rows = longs.n_chunks;
-            k_rows_warp<VEC, MAXU, IND, EPI, true><<<grid_for(b.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(b);
+            k_rows_warp<VEC, MAXU, IND, EPI, true, VF><<<grid_for(b.n_rows, TPB / 32, spmm_cap), TPB, 0, st>>>(b);
             KLAUNCH(h);
             b.n_rows = longs.n_long;
-            k_rows_combine<VEC, MAXU, EPI><<<grid_for(b.n_rows, gpb, 4 * kNumSM), TPB, 0, st>>>(b);
+            k_rows_combine<VEC, MAXU, EPI, VF><<<grid_for(b.n_rows, gpb, 4 * kNumSM), TPB, 0, st>>>(b);
         }
         KLAUNCH(h);
     }
@@ -691,7 +724,7 @@ int32_t launch_classes(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const
     return SDPLRP_OK;
 }
 
-template <bool IND, int EPI>
+template <bool IND, int EPI, bool VF = false>
 int32_t launch_csr(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const TileLayout &longs, double *sums, bool long_empty = false,
                    i64 hot_override = -1, int class_mask = 7) {
     const int r = h->r;
@@ -709,11 +742,11 @@ int32_t launch_csr(sdplrp_handle *h, RowArgs a, const RowClasses &cls, const Til
     a.Gw = (h->spmm_g0 && nv <= 16 && units == 1) ? nv : a.G;
     if (units > 4) return fail(h, SDPLRP_ERR_ARG, "rank too large for the sparse kernels (r <= 256 even / 128 odd)");
     if (vec2) {
-        if (units == 1) return launch_classes<2, 1, IND, EPI>(h, a, cls, longs, sums, long_empty, class_mask);
-        return launch_classes<2, 4, IND, EPI>(h, a, cls, longs, sums, long_empty, class_mask);
+        if (units == 1) return launch_classes<2, 1, IND, EPI, VF>(h, a, cls, longs, sums, long_empty, class_mask);
+        return launch_classes<2, 4, IND, EPI, VF>(h, a, cls, longs, sums, long_empty, class_mask);
     }
-    if (units == 1) return launch_classes<1, 1, IND, EPI>(h, a, cls, longs, sums, long_empty, class_mask);
-    return launch_classes<1, 4, IND, EPI>(h, a, cls, longs, sums, long_empty, class_mask);
+    if (units == 1) return launch_classes<1, 1, IND, EPI, VF>(h, a, cls, longs, sums, long_empty, class_mask);
+    return launch_classes<1, 4, IND, EPI, VF>(h, a, cls, longs, sums, long_empty, class_mask);
 }
 
 // mid[i] = first position of row i whose column is >= hub_cols (columns are ascending inside a row, hubs first)
@@ -900,6 +933,10 @@ int32_t grad_obj_spmm(sdplrp_handle *h, const double *X, double *Y, const double
         SDP_CHECK((launch_csr<false, 0>(h, a, h->full_cls, h->full_long, nullptr, false, hub_cols)));
         a.beg_arr = h->row_mid; a.end_arr = nullptr;  // phase two: tail columns on top, with the fused dots of the pass
         return launch_csr<false, 4>(h, a, h->full_cls, h->full_long, sums6, true, hub_cols);
+    }
+    if (obj_value_free(h)) {   // C = v * (0/1 pattern) off the diagonal, v = +-2^k: the value stream is not read
+        a.val = nullptr; a.vf_diag = h->vf_diag; a.vf_scale = h->vf_val;
+        return launch_csr<false, 2, true>(h, a, h->full_cls, h->full_long, sums6);
     }
     return launch_csr<false, 2>(h, a, h->full_cls, h->full_long, sums6);
 }

@@ -8,6 +8,8 @@
 // for a plain GEMM); everything pattern-specific is hand-written below.
 #include <cub/cub.cuh>
 #include <algorithm>
+#include <climits>
+#include <cmath>
 #include "common.cuh"
 
 namespace {
@@ -333,6 +335,29 @@ __global__ void k_cfull(i64 nnzF, const int *__restrict__ mapped, const int *__r
     for (i64 k = blockIdx.x * (i64)blockDim.x + threadIdx.x; k < nnzF; k += (i64)gridDim.x * blockDim.x) {
         const int t = mapped[i2r ? i2r[k] : k];
         cfull[k] = t >= 0 ? st[t] : 0.0;
+    }
+}
+// value-free gather pass (common.cuh: vf_val): the first off-diagonal slot of the full pattern ...
+__global__ void k_vf_first(i64 n, const int *__restrict__ ptr, const int *__restrict__ idx, int *__restrict__ first) {
+    for (i64 i = blockIdx.x * (i64)blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x)
+        for (int k = ptr[i]; k < ptr[i + 1]; k++)
+            if (idx[k] != (int)i) { atomicMin(first, k); break; }
+}
+// ... then every off-diagonal value must have v's bits, and every C_ii / v must be exact (*bad = 1 otherwise)
+__global__ void k_vf_check(i64 n, const int *__restrict__ ptr, const int *__restrict__ idx, const double *__restrict__ cfull, double v,
+                           double *__restrict__ diag, int *__restrict__ bad) {
+    const unsigned long long vb = (unsigned long long)__double_as_longlong(v);
+    for (i64 i = blockIdx.x * (i64)blockDim.x + threadIdx.x; i < n; i += (i64)gridDim.x * blockDim.x) {
+        double d = 0.0;
+        bool ok = true;
+        for (int k = ptr[i]; k < ptr[i + 1]; k++) {
+            if (idx[k] == (int)i) d = cfull[k];
+            else ok &= (unsigned long long)__double_as_longlong(cfull[k]) == vb;
+        }
+        const double q = d / v;
+        ok &= isfinite(q) && q * v == d;
+        diag[i] = q;
+        if (!ok) atomicOr(bad, 1);
     }
 }
 // mark the full-pattern slots (both mirrored positions) of every dynamic triu slot
@@ -713,7 +738,7 @@ void pre_free(sdplrp_handle *h) {
     dev_free(&h->long_mat); dev_free(&h->long_chunk_ptr); dev_free(&h->chunk_mat); dev_free(&h->chunk_part);
     dev_free(&h->triuS_static); dev_free(&h->dyn_slot); dev_free(&h->dyn_ptr); dev_free(&h->dyn_gid);
     dev_free(&h->dyn_val); dev_free(&h->dyn_pos_a); dev_free(&h->dyn_pos_b);
-    dev_free(&h->Cfull); dev_free(&h->dynS); dev_free(&h->dynrow_ptr); dev_free(&h->dynrow_col); dev_free(&h->dynrow_src);
+    dev_free(&h->Cfull); dev_free(&h->vf_diag); h->vf_val = 0.0; dev_free(&h->dynS); dev_free(&h->dynrow_ptr); dev_free(&h->dynrow_col); dev_free(&h->dynrow_src);
     dev_free(&h->dyn_diag); dev_free(&h->rowc_ptr); dev_free(&h->rowc_val); dev_free(&h->sd_flag);
     dev_free(&h->cperm); dev_free(&h->dyn_nsd_end);
     h->n_sd = 0; h->n_dyn_nsd = 0;
@@ -722,6 +747,36 @@ void pre_free(sdplrp_handle *h) {
     h->CR_valid = h->CD_valid = false;
     h->preprocessed = false;
     h->S_static_valid = false;
+}
+
+// Is C = v * (its off-diagonal pattern) + diagonal, with v = +-2^k?  (Unweighted MaxCut: v = 0.25.)  Then the gather pass
+// CD = C*D can sum the gathered rows unscaled and multiply by v once per row: scaling by a power of two commutes with
+// rounding, so the result has the same bits as the valued sum (barring subnormal or overflowing partial sums).
+static int32_t detect_value_free(sdplrp_handle *h, Tmp &tmp) {
+    cudaStream_t st = h->stream;
+    const i64 n = h->n;
+    int32_t rc = SDPLRP_OK;
+    int *flag = tmp.get<int>(h, 1, &rc);
+    if (rc) return rc;
+    const int none = INT_MAX;
+    CUDA_TRY(h, cudaMemcpyAsync(flag, &none, sizeof(int), cudaMemcpyHostToDevice, st));
+    k_vf_first<<<grid_for(n, TPB, 8 * kNumSM), TPB, 0, st>>>(n, h->full_ptr, h->full_idx, flag); KLAUNCH(h);
+    int first = none;
+    SDP_CHECK(read_int(h, flag, &first));
+    if (first == none) return SDPLRP_OK;   // diagonal C: nothing to gather
+    double v = 0.0;
+    CUDA_TRY(h, cudaMemcpyAsync(&v, h->Cfull + first, sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(h, cudaStreamSynchronize(st));
+    int ex = 0;
+    if (!std::isnormal(v) || std::fabs(std::frexp(v, &ex)) != 0.5) return SDPLRP_OK;
+    SDP_CHECK(dev_alloc(h, &h->vf_diag, n));
+    CUDA_TRY(h, cudaMemsetAsync(flag, 0, sizeof(int), st));
+    k_vf_check<<<grid_for(n, TPB, 8 * kNumSM), TPB, 0, st>>>(n, h->full_ptr, h->full_idx, h->Cfull, v, h->vf_diag, flag); KLAUNCH(h);
+    int bad = 1;
+    SDP_CHECK(read_int(h, flag, &bad));
+    if (bad) dev_free(&h->vf_diag);
+    else h->vf_val = v;
+    return SDPLRP_OK;
 }
 
 int32_t pre_build(sdplrp_handle *h, i64 n, i64 m, i64 nA, const int64_t *mat_off, const int64_t *I,
@@ -1018,6 +1073,7 @@ int32_t pre_build(sdplrp_handle *h, i64 n, i64 m, i64 nA, const int64_t *mat_off
     h->n_dynF = 0;
     if (nnzF > 0) {
         k_cfull<<<GS, TPB, 0, st>>>(nnzF, h->mapped, h->i2r, h->triuS_static, h->Cfull); KLAUNCH(h);
+        if (h->obj_mat >= 0) SDP_CHECK(detect_value_free(h, tmp));
         int *fflag = tmp.get<int>(h, nnzF + 1, &rc), *fpos = tmp.get<int>(h, nnzF + 1, &rc), *fsrc = tmp.get<int>(h, nnzF + 1, &rc);
         if (rc) return rc;
         CUDA_TRY(h, cudaMemsetAsync(fflag, 0, (size_t)(nnzF + 1) * sizeof(int), st));
