@@ -322,6 +322,27 @@ int32_t sdplrp_round_hyperplane(sdplrp_handle *h, int64_t K, const double *G, ui
 int32_t sdplrp_round_local_search(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, int64_t max_rounds,
                                   double *G_out, double *obj_round, double *obj, double *sum, int64_t *flips,
                                   int64_t *rounds, int64_t *best, double *best_x);
+/* Sweep rounding: the best threshold cut along each of K projections of R, inside a weight window.  g_k follows the
+ * rule of sdplrp_round_hyperplane (G / seed), and p_ik = <R_i, g_k> is formed with the same per-candidate FMA chain, so
+ * p_ik >= 0 is bit for bit its sign bit (-0.0 counts as +0.0).  pi_k orders the vertices by (p_ik ascending, input vertex
+ * index ascending); S_t = the first t vertices of pi_k (t = 0..n), x_t = -1 on S_t and +1 elsewhere, f_k(t) = <C, x_t x_t'>.
+ * w (n nonnegative finite weights, reference vertex order; NULL = all 1) gives W(S_t) = sum_{i in S_t} w_i, and t is
+ * feasible iff wlo <= W(S_t) <= whi.  Candidate k takes the feasible t with the smallest f_k(t), ties to the smallest t:
+ *   MaxCut / cut-norm:  w = NULL, wlo = -inf, whi = +inf (contains the hyperplane cut t = #(p_k < 0));
+ *   exact bisection:    w = NULL, wlo = floor(n/2), whi = ceil(n/2);
+ *   mu-balanced cut:    w = degrees, wlo = mu vol, whi = (1 - mu) vol.
+ * Outputs per candidate: thresh[k] = t_k, or -1 when no t is feasible (then obj[k] = +inf, sum[k] = wS[k] = NaN);
+ * obj[k] = <C, x x'> of the chosen vector evaluated like sdplrp_round_hyperplane's obj; sum[k] = n - 2 t_k;
+ * wS[k] = W(S_{t_k}).  best (1-based) is the smallest obj, ties to the lowest k; best_x (reference order, +-1.0) its vector,
+ * best_profile (n + 1) its f(0..n) as the scan computed it, best_order (n, 1-based input vertex ids) its order pi.
+ * Every output except obj and best may be NULL.  Candidate k's result does not depend on K, the vertex order or the GPU
+ * count.  Reads R only, like sdplrp_round_hyperplane.
+ * Several GPUs: every rank passes the same K, seed, G, w, wlo and whi and receives the same results.
+ * Errors as sdplrp_round_hyperplane, and SDPLRP_ERR_ARG for wlo > whi, a NaN bound, a negative or non-finite weight, and
+ * when no threshold of any candidate is feasible. */
+int32_t sdplrp_round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, const double *w, double wlo,
+                           double whi, double *G_out, double *obj, double *sum, double *wS, int64_t *thresh,
+                           int64_t *best, double *best_x, double *best_profile, int64_t *best_order);
 
 /* ---- native host driver (SURVEY.md 8f, f1) ------------------------------ */
 /* BurerMonteiroConfig (src/options.jl:1-24); every field is 8 bytes wide so the layout is the same from C, Julia

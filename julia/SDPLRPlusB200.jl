@@ -398,6 +398,32 @@ function round_local_search(aux::B200Auxiliary, K::Integer; r::Integer, G=nothin
     return obj0, obj, tot, flips, rounds, Int(best[]), x, G_used
 end
 
+"""
+    round_sweep(aux, K; r, G = nothing, seed = 0, w = nothing, window = (-Inf, Inf))
+        -> (obj, sum, wS, thresh, best, best_x, best_profile, best_order, G_used)
+
+Sweep rounding on the device: for each direction g_k of `round_hyperplane` the vertices are ordered by (<R_i, g_k>, vertex
+index) and the prefix cut S_t (x = -1 on the first t vertices) with the smallest <C, xx'> whose weight sum(w[S_t]) lies
+in `window` is kept (`w = nothing`: unit weights; exact bisection: `window = (n ÷ 2, cld(n, 2))`).  `thresh[k]` is t
+(-1 when no prefix fits, with obj[k] = Inf), `wS[k]` its weight, `sum[k] = n - 2t`; `best` (1-based) the smallest obj,
+`best_x` its +-1 vector, `best_profile` its objective at every t = 0..n and `best_order` its order (1-based vertex ids).
+Reads R only.
+"""
+function round_sweep(aux::B200Auxiliary, K::Integer; r::Integer, G=nothing, seed=0, w=nothing, window=(-Inf, Inf))
+    Gin = G === nothing ? Ptr{Float64}(C_NULL) : Matrix{Float64}(G)
+    G === nothing || size(Gin) == (r, K) || throw(ArgumentError("G must be r x K"))
+    win = w === nothing ? Ptr{Float64}(C_NULL) : Vector{Float64}(w)
+    w === nothing || length(win) == aux.n || throw(ArgumentError("w must have n entries"))
+    G_used = zeros(r, K); obj = zeros(K); tot = zeros(K); wS = zeros(K); thresh = zeros(Int64, K); best = Ref{Int64}(0)
+    x = zeros(aux.n); prof = zeros(aux.n + 1); order = zeros(Int64, aux.n)
+    GC.@preserve Gin win G_used obj tot wS thresh x prof order check(aux.h, ccall((:sdplrp_round_sweep, LIB), Int32,
+        (Ptr{Cvoid}, Int64, Ptr{Float64}, UInt64, Ptr{Float64}, Float64, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Int64}, Ref{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+        aux.h.ptr, K, Gin, UInt64(seed), win, Float64(window[1]), Float64(window[2]), G_used, obj, tot, wS, thresh, best, x,
+        prof, order))
+    return obj, tot, wS, thresh, Int(best[]), x, prof, order, G_used
+end
+
 function apply_kwargs!(config, kwargs)
     for (k, v) in kwargs
         hasfield(BurerMonteiroConfig, Symbol(k)) ? setfield!(config, Symbol(k), v) : @error "Unrecognized keyword argument $k"

@@ -7,6 +7,7 @@ import fails loudly, and on a machine without a CUDA device `Handle()` raises.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -118,6 +119,8 @@ _SIGNATURES.update({
     "sdplrp_round_hyperplane": [_H, C.c_int64, _p_f64, C.c_uint64, _p_f64, _p_f64, _p_f64, _p_i64, _p_f64],
     "sdplrp_round_local_search": [_H, C.c_int64, _p_f64, C.c_uint64, C.c_int64, _p_f64, _p_f64, _p_f64, _p_f64, _p_i64, _p_i64, _p_i64,
                                   _p_f64],
+    "sdplrp_round_sweep": [_H, C.c_int64, _p_f64, C.c_uint64, _p_f64, C.c_double, C.c_double, _p_f64, _p_f64, _p_f64, _p_f64, _p_i64,
+                           _p_i64, _p_f64, _p_f64, _p_i64],
 })
 
 _SPECIAL = {
@@ -564,6 +567,33 @@ class Handle:
             C.byref(best), x.ctypes.data_as(_p_f64)))
         return {"obj_round": obj0, "obj": obj, "sum": tot, "flips": flips, "rounds": rounds, "best": best.value - 1, "best_x": x,
                 "G_used": G_used}
+
+    def round_sweep(self, K, G=None, seed=0, w=None, window=(-math.inf, math.inf)):
+        """sdplrp_round_sweep: for each of the K projections p_k = R g_k of round_hyperplane, the best threshold cut of the
+        sweep order (p_k ascending, then input vertex index) whose weight W(S_t) = sum of w over the t first vertices lies in
+        `window` (w None: unit weights) -> dict(obj (K,; inf when no threshold is feasible), sum (K,) = n - 2 thresh,
+        wS (K,), thresh (K,; -1 = none feasible), best (0-based), best_x (n,) of +-1.0, best_profile (n + 1,) = f(0..n) of the
+        best candidate, best_order (n,) its sweep order as 0-based input vertex ids, G_used (K, r))"""
+        K = int(K)
+        pg = None
+        if G is not None:
+            G, pg = _f64(G)
+            assert G.size == K * self.r, (G.shape, K, self.r)
+        pw = None
+        if w is not None:
+            w, pw = _f64(w)
+            assert w.size == self.n, (w.shape, self.n)
+        wlo, whi = (float(v) for v in window)
+        G_used = np.empty((K, self.r), np.float64)
+        obj, tot, wS, x, prof = np.empty(K), np.empty(K), np.empty(K), np.empty(self.n), np.empty(self.n + 1)
+        thresh, order = np.empty(K, np.int64), np.empty(self.n, np.int64)
+        best = C.c_int64()
+        self._check(self.lib.sdplrp_round_sweep(
+            self._h, K, pg, int(seed), pw, wlo, whi, G_used.ctypes.data_as(_p_f64), obj.ctypes.data_as(_p_f64),
+            tot.ctypes.data_as(_p_f64), wS.ctypes.data_as(_p_f64), thresh.ctypes.data_as(_p_i64), C.byref(best),
+            x.ctypes.data_as(_p_f64), prof.ctypes.data_as(_p_f64), order.ctypes.data_as(_p_i64)))
+        return {"obj": obj, "sum": tot, "wS": wS, "thresh": thresh, "best": best.value - 1, "best_x": x, "best_profile": prof,
+                "best_order": order - 1, "G_used": G_used}
 
     def solve(self, cfg, r, Rt0=None, lambda0=None, normb=1.0, normC=1.0):
         """sdplrp_solve: the native outer loop -> (Result, best_lambda[m+1])"""

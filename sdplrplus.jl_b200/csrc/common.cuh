@@ -100,6 +100,17 @@ struct RoundingState {
     int *seg_row = nullptr, *seg_start = nullptr;         // n_seg: row and first nonzero of every segment
     double *seg_part = nullptr;                           // n_seg x 64 want sums of a segment
     long long n_seg = 0, l_lo = 0, l_hi = 0, s_lo = 0, s_hi = 0;  // the owned long rows [l_lo, l_hi) and their segments [s_lo, s_hi)
+    // sweep rounding (first use; the segments above are shared)
+    double *sw_P = nullptr, *sw_delta = nullptr;          // n x 16: projections / move deltas of the batch (internal order)
+    int *sw_order = nullptr;                              // 16 x n: sweep order of every candidate (internal ids)
+    unsigned long long *sw_keys = nullptr;                // 2 x n: radix sort keys (in, out); also the order download buffer
+    int *sw_vals = nullptr;                               // n: radix sort values in
+    unsigned char *sw_cub = nullptr;                      // radix sort scratch
+    size_t sw_cub_bytes = 0;
+    double *sw_tiles = nullptr;                           // 16 x ntiles x 5: tile sums -> offsets (2), tile minima (3)
+    long long sw_ntiles = 0;
+    double *sw_w = nullptr;                               // n: vertex weights (internal order)
+    double *sw_prof = nullptr;                            // n + 1: f(0..n) of the best candidate
 };
 
 struct LowRank {

@@ -20,9 +20,18 @@
 //               rows, and a flipped row marks itself and its neighbours dirty (identical byte stores).
 // Rows with more than kLsLong nonzeros are cut into segments of kLsSeg nonzeros, one CTA each; the want sums of a long row
 // are combined over its segments in a fixed order.
+//
+// Sweep rounding (sdplrp_round_sweep) goes in batches of kSweepB = 16 candidates, one 128-byte row of projections per vertex:
+// projection pass (k_round_sign<16, true>) -> per candidate a stable radix sort of (key, input id) -> delta pass (k_sw_delta*,
+// the move deltas along each order) -> three-phase tile scan and selection (k_sw_tile_sums, k_sw_tile_scan, k_sw_scan,
+// k_sw_select) -> words of the chosen prefixes (k_sw_words) -> evaluation pass.  DESIGN.md §3f.
 // Nothing outside the rounding buffers (h->rnd) and the reduction scratch is written.
+#include <limits.h>
 #include <math.h>
+#include <string.h>
 #include <algorithm>
+#include <cmath>
+#include <cub/cub.cuh>
 #include <vector>
 #include "common.cuh"
 
@@ -35,6 +44,11 @@ constexpr int kEvalChunk = 32;     // nonzeros per thread chunk of the evaluatio
 constexpr int kLsTPB = 128;
 constexpr int kLsLong = 128;       // local search: rows with more nonzeros than this go to the segment kernels
 constexpr int kLsSeg = 4096;       // nonzeros per segment (one CTA) of a long row
+constexpr int kSweepB = 16;        // sweep rounding: candidates per batch (a vertex's projections are one 128-byte row)
+constexpr int kSwTPB = 256;        // sweep scan: threads per tile
+constexpr int kSwItems = 16;       // consecutive sweep positions per thread
+constexpr int kSwTile = kSwTPB * kSwItems;
+constexpr int kSwSel = 5;          // per candidate: f(t), t (-1: none feasible), W(S_t), boundary projection, boundary input id
 typedef unsigned long long Word;
 
 __host__ __device__ inline unsigned long long mix64(unsigned long long x) {
@@ -59,18 +73,22 @@ __device__ __forceinline__ void counts_to_values(const unsigned (&cnt)[2], int l
     for (int k = 0; k < kRoundB; k++) v[k] = lane == (k & 31) ? (double)cnt[k >> 5] : 0.0;
 }
 
-// words[i] bit k = (<R_i, g_k> >= 0) for the owned rows; cnt[k] = number of set bits over them (k < 64)
+// words[i] bit k = (<R_i, g_k> >= 0) for the owned rows; cnt[k] = number of set bits over them (k < 64).
+// PROJ (sweep rounding, NB = kSweepB): proj[i * NB + k] = <R_i, g_k> (-0.0 stored as +0.0, 0 for k >= nb) instead of the
+// bits, no counts.  The per-candidate FMA chain is the same in both forms, so proj >= 0 is bit for bit the sign bit.
+template <int NB, bool PROJ>
 __global__ void __launch_bounds__(kSignTPB) k_round_sign(i64 row_lo, i64 nrows, int r, const double *__restrict__ R,
                                                           const double *__restrict__ G, int nb, Word *__restrict__ words,
-                                                          double *partials, unsigned *ticket, double *cnt_out) {
-    __shared__ double Gs[kSignCols][kRoundB];
+                                                          double *__restrict__ proj, double *partials, unsigned *ticket,
+                                                          double *cnt_out) {
+    __shared__ double Gs[kSignCols][NB];
     const int lane = threadIdx.x & 31;
     unsigned cnt[2] = {0u, 0u};  // candidates lane and lane + 32 of this warp
     const bool single = r <= kSignCols;
     auto load_cols = [&](int c0) {
         const int nc = min(kSignCols, r - c0);
-        for (int e = threadIdx.x; e < kSignCols * kRoundB; e += blockDim.x) {
-            const int c = e / kRoundB, k = e - c * kRoundB;
+        for (int e = threadIdx.x; e < kSignCols * NB; e += blockDim.x) {
+            const int c = e / NB, k = e - c * NB;
             Gs[c][k] = (c < nc && k < nb) ? G[(size_t)k * r + c0 + c] : 0.0;
         }
     };
@@ -79,9 +97,9 @@ __global__ void __launch_bounds__(kSignTPB) k_round_sign(i64 row_lo, i64 nrows, 
         const i64 i = base + threadIdx.x;
         const bool valid = i < nrows;
         const double *Ri = R + (size_t)(row_lo + (valid ? i : 0)) * r;
-        double acc[kRoundB];
+        double acc[NB];
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) acc[k] = 0.0;
+        for (int k = 0; k < NB; k++) acc[k] = 0.0;
         for (int c0 = 0; c0 < r; c0 += kSignCols) {
             if (!single) { __syncthreads(); load_cols(c0); __syncthreads(); }
             const int nc = min(kSignCols, r - c0);
@@ -89,23 +107,33 @@ __global__ void __launch_bounds__(kSignTPB) k_round_sign(i64 row_lo, i64 nrows, 
                 for (int c = 0; c < nc; c++) {
                     const double x = Ri[c0 + c];
 #pragma unroll
-                    for (int k = 0; k < kRoundB; k++) acc[k] = fma(x, Gs[c][k], acc[k]);
+                    for (int k = 0; k < NB; k++) acc[k] = fma(x, Gs[c][k], acc[k]);
                 }
             }
         }
-        Word w = 0ull;
+        if constexpr (PROJ) {
+            if (valid) {
+                double2 *Pi = reinterpret_cast<double2 *>(proj + (size_t)(row_lo + i) * NB);
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) w |= (Word)(acc[k] >= 0.0) << k;
-        if (!valid) w = 0ull;
-        else words[row_lo + i] = w;
-        ballot_counts(w, lane, cnt);
+                for (int k = 0; k < NB; k += 2) Pi[k / 2] = make_double2(acc[k] + 0.0, acc[k + 1] + 0.0);
+            }
+        } else {
+            Word w = 0ull;
+#pragma unroll
+            for (int k = 0; k < NB; k++) w |= (Word)(acc[k] >= 0.0) << k;
+            if (!valid) w = 0ull;
+            else words[row_lo + i] = w;
+            ballot_counts(w, lane, cnt);
+        }
     }
-    double v[kRoundB];
-    counts_to_values(cnt, lane, v);
-    grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
+    if constexpr (!PROJ) {
+        double v[kRoundB];
+        counts_to_values(cnt, lane, v);
+        grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) if (k < nb) cnt_out[k] = s[k];
-    });
+            for (int k = 0; k < kRoundB; k++) if (k < nb) cnt_out[k] = s[k];
+        });
+    }
 }
 
 // first owned row of every chunk of kEvalChunk nonzeros (chunk c starts at nonzero e_lo + c * kEvalChunk)
@@ -391,6 +419,316 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_count(i64 row_lo, i64 nrows, cons
     });
 }
 
+// ---- sweep rounding --------------------------------------------------------------------------------------------------
+// Candidate k orders the vertices by (p_ik, input id) ascending; S_t = the first t of them.  Vertex j comes after v in that
+// order iff (p_jk, ref_j) > (p_vk, ref_v); the input ids are read only where projections are equal.
+__device__ __forceinline__ int sw_ref(const int *__restrict__ iperm, i64 i) { return iperm ? iperm[i] : (int)i; }
+
+__device__ __forceinline__ void sw_load_row(const double *__restrict__ P, i64 i, double (&p)[kSweepB]) {
+    const double2 *row = reinterpret_cast<const double2 *>(P + (size_t)i * kSweepB);
+#pragma unroll
+    for (int k = 0; k < kSweepB; k += 2) { const double2 t = __ldg(row + k / 2); p[k] = t.x; p[k + 1] = t.y; }
+}
+
+// acc[k] += C_vj when j comes after v in candidate k's order, -= C_vj when before (k < nb: mask = low nb bits)
+__device__ __forceinline__ void sw_accumulate(const double *__restrict__ P, const int *__restrict__ iperm, int j, double v,
+                                              const double (&pv)[kSweepB], int rv, unsigned mask, double (&acc)[kSweepB]) {
+    double pj[kSweepB];
+    sw_load_row(P, j, pj);
+    unsigned gt = 0u, eq = 0u;
+#pragma unroll
+    for (int k = 0; k < kSweepB; k++) { gt |= (unsigned)(pj[k] > pv[k]) << k; eq |= (unsigned)(pj[k] == pv[k]) << k; }
+    eq &= mask;
+    if (eq && sw_ref(iperm, j) > rv) gt |= eq;
+#pragma unroll
+    for (int k = 0; k < kSweepB; k++) acc[k] += ((gt >> k) & 1u) ? v : -v;
+}
+
+// sort input of candidate k in input vertex order: keys[u] = order-preserving bits of p_{perm(u)k}, vals[u] = perm(u)
+__global__ void k_sw_keys(i64 n, int k, const double *__restrict__ P, const int *__restrict__ perm, Word *__restrict__ keys,
+                          int *__restrict__ vals) {
+    for (i64 u = blockIdx.x * (i64)blockDim.x + threadIdx.x; u < n; u += (i64)gridDim.x * blockDim.x) {
+        const int i = perm ? perm[u] : (int)u;
+        const Word b = (Word)__double_as_longlong(P[(size_t)i * kSweepB + k]);
+        keys[u] = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+        vals[u] = i;
+    }
+}
+
+// delta pass, rows with at most kLsLong nonzeros: one thread per owned row, delta[v][k] = -4 (sum_after C_vj - sum_before C_vj)
+__global__ void __launch_bounds__(kLsTPB) k_sw_delta(i64 row_lo, i64 row_hi, const int *__restrict__ ptr, const int *__restrict__ idx,
+                                                    const double *__restrict__ val, const double *__restrict__ P,
+                                                    const int *__restrict__ iperm, unsigned mask, double *__restrict__ delta) {
+    for (i64 i = row_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; i < row_hi; i += (i64)gridDim.x * blockDim.x) {
+        const int a = ptr[i], b = ptr[i + 1];
+        if (b - a > kLsLong) continue;
+        double pv[kSweepB], acc[kSweepB];
+        sw_load_row(P, i, pv);
+        const int rv = sw_ref(iperm, i);
+#pragma unroll
+        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
+        for (int e = a; e < b; e++) {
+            const int j = idx[e];
+            const double v = val[e];
+            if (j == i || v == 0.0) continue;
+            sw_accumulate(P, iperm, j, v, pv, rv, mask, acc);
+        }
+        double2 *out = reinterpret_cast<double2 *>(delta + (size_t)i * kSweepB);
+#pragma unroll
+        for (int k = 0; k < kSweepB; k += 2) out[k / 2] = make_double2(-4.0 * acc[k], -4.0 * acc[k + 1]);
+    }
+}
+
+// delta pass, long rows: one CTA per segment of an owned long row; part[s][k] = the segment's signed sums (fixed-order CTA sum)
+__global__ void __launch_bounds__(kLsTPB) k_sw_delta_seg(i64 s_lo, i64 s_hi, const int *__restrict__ seg_row,
+                                                        const int *__restrict__ seg_start, const int *__restrict__ ptr,
+                                                        const int *__restrict__ idx, const double *__restrict__ val,
+                                                        const double *__restrict__ P, const int *__restrict__ iperm, unsigned mask,
+                                                        double *__restrict__ part) {
+    for (i64 s = s_lo + blockIdx.x; s < s_hi; s += gridDim.x) {
+        const int i = seg_row[s];
+        const int e0 = seg_start[s], e1 = min(e0 + kLsSeg, ptr[i + 1]);
+        double pv[kSweepB], acc[kSweepB];
+        sw_load_row(P, i, pv);
+        const int rv = sw_ref(iperm, i);
+#pragma unroll
+        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
+        for (int e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
+            const int j = idx[e];
+            const double v = val[e];
+            if (j == i || v == 0.0) continue;
+            sw_accumulate(P, iperm, j, v, pv, rv, mask, acc);
+        }
+        block_sum<kSweepB>(acc);
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int k = 0; k < kSweepB; k++) part[(size_t)s * kSweepB + k] = acc[k];
+        }
+    }
+}
+
+// delta pass, long rows: the segment sums of every owned long row added in segment order
+__global__ void k_sw_delta_combine(i64 l_lo, i64 l_hi, const int *__restrict__ long_rows, const int *__restrict__ long_sptr,
+                                   const double *__restrict__ part, double *__restrict__ delta) {
+    for (i64 L = l_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; L < l_hi; L += (i64)gridDim.x * blockDim.x) {
+        double acc[kSweepB];
+#pragma unroll
+        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
+        for (int s = long_sptr[L]; s < long_sptr[L + 1]; s++) {
+#pragma unroll
+            for (int k = 0; k < kSweepB; k++) acc[k] += part[(size_t)s * kSweepB + k];
+        }
+        double *out = delta + (size_t)long_rows[L] * kSweepB;
+#pragma unroll
+        for (int k = 0; k < kSweepB; k++) out[k] = -4.0 * acc[k];
+    }
+}
+
+// exclusive prefix of (a, b) over the threads of the CTA in thread order (shuffle scans: the same bits every run)
+__device__ __forceinline__ void sw_block_exscan(double &a, double &b) {
+    __shared__ double ws[2][32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    double ia = a, ib = b;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const double ta = __shfl_up_sync(0xffffffffu, ia, o), tb = __shfl_up_sync(0xffffffffu, ib, o);
+        if (lane >= o) { ia += ta; ib += tb; }
+    }
+    double ea = __shfl_up_sync(0xffffffffu, ia, 1), eb = __shfl_up_sync(0xffffffffu, ib, 1);
+    if (lane == 0) { ea = 0.0; eb = 0.0; }
+    __syncthreads();   // ws reused across calls
+    if (lane == 31) { ws[0][wid] = ia; ws[1][wid] = ib; }
+    __syncthreads();
+    if (wid == 0) {
+        double xa = lane < nw ? ws[0][lane] : 0.0, xb = lane < nw ? ws[1][lane] : 0.0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double ta = __shfl_up_sync(0xffffffffu, xa, o), tb = __shfl_up_sync(0xffffffffu, xb, o);
+            if (lane >= o) { xa += ta; xb += tb; }
+        }
+        double pa = __shfl_up_sync(0xffffffffu, xa, 1), pb = __shfl_up_sync(0xffffffffu, xb, 1);
+        if (lane == 0) { pa = 0.0; pb = 0.0; }
+        if (lane < nw) { ws[0][lane] = pa; ws[1][lane] = pb; }
+    }
+    __syncthreads();
+    a = ws[0][wid] + ea;
+    b = ws[1][wid] + eb;
+}
+
+// (f, t, W) minimum over the CTA: smallest f, ties to the smallest t (t = INT64_MAX: none).  Exact comparisons only, so the
+// result does not depend on the order.  Valid in thread 0.
+__device__ __forceinline__ bool sw_better(double f, long long t, double bf, long long bt) { return f < bf || (f == bf && t < bt); }
+
+__device__ __forceinline__ void sw_block_argmin(double &f, long long &t, double &w) {
+    __shared__ double sf[32], sw[32];
+    __shared__ long long st[32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double of = __shfl_xor_sync(0xffffffffu, f, o), ow = __shfl_xor_sync(0xffffffffu, w, o);
+        const long long ot = __shfl_xor_sync(0xffffffffu, t, o);
+        if (sw_better(of, ot, f, t)) { f = of; t = ot; w = ow; }
+    }
+    __syncthreads();
+    if (lane == 0) { sf[wid] = f; st[wid] = t; sw[wid] = w; }
+    __syncthreads();
+    if (wid == 0) {
+        f = lane < nw ? sf[lane] : INFINITY;
+        t = lane < nw ? st[lane] : LLONG_MAX;
+        w = lane < nw ? sw[lane] : 0.0;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const double of = __shfl_xor_sync(0xffffffffu, f, o), ow = __shfl_xor_sync(0xffffffffu, w, o);
+            const long long ot = __shfl_xor_sync(0xffffffffu, t, o);
+            if (sw_better(of, ot, f, t)) { f = of; t = ot; w = ow; }
+        }
+    }
+}
+
+// scan phase 1, grid (tiles, candidates): tsum[k][tile] = the tile's sums of delta and w along candidate k's order
+__global__ void __launch_bounds__(kSwTPB) k_sw_tile_sums(i64 n, i64 ntiles, const int *__restrict__ order, const double *__restrict__ delta,
+                                                        const double *__restrict__ w, double *__restrict__ tsum_d,
+                                                        double *__restrict__ tsum_w) {
+    const int k = blockIdx.y;
+    const int *ord = order + (size_t)k * n;
+    const i64 base = (i64)blockIdx.x * kSwTile;
+    double v[2] = {0.0, 0.0};
+    for (int q = 0; q < kSwItems; q++) {
+        const i64 s = base + q * kSwTPB + threadIdx.x;
+        if (s < n) {
+            const int u = ord[s];
+            v[0] += delta[(size_t)u * kSweepB + k];
+            v[1] += w ? w[u] : 1.0;
+        }
+    }
+    block_sum<2>(v);
+    if (threadIdx.x == 0) { tsum_d[(size_t)k * ntiles + blockIdx.x] = v[0]; tsum_w[(size_t)k * ntiles + blockIdx.x] = v[1]; }
+}
+
+// scan phase 2, one CTA per candidate: the tile sums replaced by their exclusive prefix, in tile order
+__global__ void __launch_bounds__(kSwTPB) k_sw_tile_scan(i64 ntiles, double *__restrict__ tsum_d, double *__restrict__ tsum_w) {
+    double *d = tsum_d + (size_t)blockIdx.x * ntiles, *w = tsum_w + (size_t)blockIdx.x * ntiles;
+    __shared__ double carry[2];
+    if (threadIdx.x == 0) { carry[0] = 0.0; carry[1] = 0.0; }
+    __syncthreads();
+    for (i64 t0 = 0; t0 < ntiles; t0 += kSwTPB) {
+        const i64 t = t0 + threadIdx.x;
+        const double a0 = t < ntiles ? d[t] : 0.0, b0 = t < ntiles ? w[t] : 0.0;
+        double a = a0, b = b0;
+        sw_block_exscan(a, b);
+        const double ca = carry[0], cb = carry[1];
+        if (t < ntiles) { d[t] = ca + a; w[t] = cb + b; }
+        __syncthreads();
+        if (threadIdx.x == kSwTPB - 1) { carry[0] = ca + (a + a0); carry[1] = cb + (b + b0); }
+        __syncthreads();
+    }
+}
+
+// scan phase 3, grid (tiles, candidates): the tile rescanned from its offset.  Position s adds delta / w of vertex
+// order[s]: f(s + 1) = sum(C) + prefix, W(S_{s+1}) = prefix of w.  The feasible minimum of the tile (ties to the smallest t)
+// goes to tbest; prof (candidate 0 only, may be NULL) receives f(0..n).
+__global__ void __launch_bounds__(kSwTPB) k_sw_scan(i64 n, i64 ntiles, const int *__restrict__ order, const double *__restrict__ delta,
+                                                   const double *__restrict__ w, const double *__restrict__ toff_d,
+                                                   const double *__restrict__ toff_w, const double *__restrict__ csum, double wlo,
+                                                   double whi, double *__restrict__ prof, double *__restrict__ tbest) {
+    __shared__ int ids[kSwTile];
+    const int k = blockIdx.y;
+    const int *ord = order + (size_t)k * n;
+    const i64 base = (i64)blockIdx.x * kSwTile;
+    for (int q = 0; q < kSwItems; q++) {
+        const i64 s = base + q * kSwTPB + threadIdx.x;
+        ids[q * kSwTPB + threadIdx.x] = s < n ? ord[s] : -1;
+    }
+    __syncthreads();
+    double dl[kSwItems], wl[kSwItems], a = 0.0, b = 0.0;
+#pragma unroll
+    for (int q = 0; q < kSwItems; q++) {
+        const int u = ids[threadIdx.x * kSwItems + q];
+        dl[q] = u >= 0 ? delta[(size_t)u * kSweepB + k] : 0.0;
+        wl[q] = u >= 0 ? (w ? w[u] : 1.0) : 0.0;
+        a += dl[q];
+        b += wl[q];
+    }
+    sw_block_exscan(a, b);
+    const size_t tk = (size_t)k * ntiles + blockIdx.x;
+    double pd = toff_d[tk] + a, pw = toff_w[tk] + b;
+    const double c = *csum;
+    double bf = INFINITY, bw = 0.0;
+    long long bt = LLONG_MAX;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {   // t = 0: S empty
+        if (prof) prof[0] = c;
+        if (wlo <= 0.0 && 0.0 <= whi) { bf = c; bt = 0; }
+    }
+#pragma unroll
+    for (int q = 0; q < kSwItems; q++) {
+        const i64 s = base + (i64)threadIdx.x * kSwItems + q;
+        if (s < n) {
+            pd += dl[q];
+            pw += wl[q];
+            const double f = c + pd;
+            if (prof) prof[s + 1] = f;
+            if (wlo <= pw && pw <= whi && f < bf) { bf = f; bt = s + 1; bw = pw; }
+        }
+    }
+    sw_block_argmin(bf, bt, bw);
+    if (threadIdx.x == 0) {
+        double *o = tbest + tk * 3;
+        o[0] = bf; o[1] = (double)bt; o[2] = bw;
+    }
+}
+
+// selection, one CTA per candidate: the minimum over the tiles, and the boundary vertex b = order[t] whose (p, input id)
+// starts the +1 side (t = n: none, every x = -1; no feasible t: every x = +1, the candidate is reported infeasible)
+__global__ void __launch_bounds__(kSwTPB) k_sw_select(i64 n, i64 ntiles, const double *__restrict__ tbest, const int *__restrict__ order,
+                                                     const double *__restrict__ P, const int *__restrict__ iperm,
+                                                     double *__restrict__ sel) {
+    const int k = blockIdx.x;
+    double bf = INFINITY, bw = 0.0;
+    long long bt = LLONG_MAX;
+    for (i64 tile = threadIdx.x; tile < ntiles; tile += blockDim.x) {
+        const double *o = tbest + ((size_t)k * ntiles + tile) * 3;
+        const long long t = o[1] >= 9.0e18 ? LLONG_MAX : (long long)o[1];
+        if (sw_better(o[0], t, bf, bt)) { bf = o[0]; bt = t; bw = o[2]; }
+    }
+    sw_block_argmin(bf, bt, bw);
+    if (threadIdx.x == 0) {
+        double *o = sel + (size_t)k * kSwSel;
+        const bool none = bt == LLONG_MAX;
+        o[0] = bf;
+        o[1] = none ? -1.0 : (double)bt;
+        o[2] = bw;
+        if (none) { o[3] = -INFINITY; o[4] = -1.0; }
+        else if (bt == n) { o[3] = INFINITY; o[4] = 0.0; }
+        else { const int u = order[(size_t)k * n + bt]; o[3] = P[(size_t)u * kSweepB + k]; o[4] = (double)sw_ref(iperm, u); }
+    }
+}
+
+// words of the owned rows: bit k set (x = +1) iff (p_ik, input id) >= the boundary of candidate k
+__global__ void k_sw_words(i64 row_lo, i64 row_hi, const double *__restrict__ P, const int *__restrict__ iperm,
+                           const double *__restrict__ sel, int nb, Word *__restrict__ words) {
+    __shared__ double bp[kSweepB], bi[kSweepB];
+    if (threadIdx.x < kSweepB) {
+        bp[threadIdx.x] = threadIdx.x < nb ? sel[threadIdx.x * kSwSel + 3] : INFINITY;
+        bi[threadIdx.x] = threadIdx.x < nb ? sel[threadIdx.x * kSwSel + 4] : 0.0;
+    }
+    __syncthreads();
+    for (i64 i = row_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; i < row_hi; i += (i64)gridDim.x * blockDim.x) {
+        double p[kSweepB];
+        sw_load_row(P, i, p);
+        const double ri = (double)sw_ref(iperm, i);
+        Word w = 0ull;
+#pragma unroll
+        for (int k = 0; k < kSweepB; k++) w |= (Word)(p[k] > bp[k] || (p[k] == bp[k] && ri >= bi[k])) << k;
+        words[i] = w;
+    }
+}
+
+// out[s] = 1-based input id of the vertex at sweep position s
+__global__ void k_sw_order_out(i64 n, const int *__restrict__ order, const int *__restrict__ iperm, int64_t *__restrict__ out) {
+    for (i64 s = blockIdx.x * (i64)blockDim.x + threadIdx.x; s < n; s += (i64)gridDim.x * blockDim.x)
+        out[s] = (int64_t)sw_ref(iperm, order[s]) + 1;
+}
+
 // standard normal keyed by (seed, candidate, column) (counter-based hash + Box-Muller): independent of K, of the vertex
 // order and of the number of GPUs
 double hyperplane_normal(unsigned long long seed, i64 k, i64 c) {
@@ -433,8 +771,8 @@ int32_t ensure_problem_buffers(sdplrp_handle *h) {
 
 int32_t sign_pass(sdplrp_handle *h, const double *dG, int nb, double *cnt_out) {
     const i64 nrows = h->row_hi - h->row_lo;
-    k_round_sign<<<grid_for(std::max<i64>(nrows, 1), kSignTPB, 2 * kRedBlocks), kSignTPB, 0, h->stream>>>(
-        h->row_lo, nrows, h->r, h->R, dG, nb, h->rnd.words, h->partials, h->ticket, cnt_out);
+    k_round_sign<kRoundB, false><<<grid_for(std::max<i64>(nrows, 1), kSignTPB, 2 * kRedBlocks), kSignTPB, 0, h->stream>>>(
+        h->row_lo, nrows, h->r, h->R, dG, nb, h->rnd.words, nullptr, h->partials, h->ticket, cnt_out);
     KLAUNCH(h);
     CUDA_TRY(h, cudaGetLastError());
     return SDPLRP_OK;
@@ -460,11 +798,11 @@ int32_t upload(sdplrp_handle *h, T **dst, const std::vector<T> &src) {
     return SDPLRP_OK;
 }
 
-// local-search buffers (first use after preprocessing): want / flip / best words and dirty flags (n each), and the segments
-// of the rows of the full pattern with more than kLsLong nonzeros (all rows: the apply pass covers every row on every rank)
-int32_t ensure_search_buffers(sdplrp_handle *h) {
+// the segments of the rows of the full pattern with more than kLsLong nonzeros (all rows: the apply pass of the local search
+// covers every row on every rank), and their partial sums (first use after preprocessing)
+int32_t ensure_segments(sdplrp_handle *h) {
     RoundingState &s = h->rnd;
-    if (s.want) return SDPLRP_OK;
+    if (s.seg_part) return SDPLRP_OK;
     const i64 n = h->n;
     std::vector<int> ptr((size_t)n + 1), long_rows, long_sptr(1, 0), seg_row, seg_start;
     CUDA_TRY(h, cudaMemcpyAsync(ptr.data(), h->full_ptr, ptr.size() * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
@@ -487,6 +825,15 @@ int32_t ensure_search_buffers(sdplrp_handle *h) {
     SDP_CHECK(upload(h, &s.seg_start, seg_start));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     SDP_CHECK(dev_alloc(h, &s.seg_part, s.n_seg * kRoundB));
+    return SDPLRP_OK;
+}
+
+// local-search buffers (first use after preprocessing): the segments, want / flip / best words and dirty flags (n each)
+int32_t ensure_search_buffers(sdplrp_handle *h) {
+    RoundingState &s = h->rnd;
+    if (s.want) return SDPLRP_OK;
+    const i64 n = h->n;
+    SDP_CHECK(ensure_segments(h));
     SDP_CHECK(dev_alloc(h, &s.flip, n));
     SDP_CHECK(dev_alloc(h, &s.best_words, n));
     SDP_CHECK(dev_alloc(h, &s.dirty, n));
@@ -561,28 +908,43 @@ constexpr int kSumBlock = 4 * kRoundB;
 
 // K candidates in batches of 64: sign pass, all-gather of the words, evaluation pass and, when `search`, the one-flip
 // descent and a second evaluation pass.  sdplrp_round_hyperplane is the case without search.
-int32_t round_batches(sdplrp_handle *h, const char *name, int64_t K, const double *G, uint64_t seed, bool search, int64_t max_rounds,
-                      double *G_out, double *obj_round, double *obj, double *sum, int64_t *flips, int64_t *rounds, int64_t *best,
-                      double *best_x) {
+// the checks every rounding entry point makes before it touches the device
+int32_t rounding_check(sdplrp_handle *h, const char *name, int64_t K, const void *obj, const void *best) {
     if (!h->preprocessed) return fail(h, SDPLRP_ERR_STATE, "call sdplrp_preprocess first");
     if (h->r <= 0) return fail(h, SDPLRP_ERR_STATE, "call sdplrp_set_rank first");
     if (K < 1 || !obj || !best) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": K >= 1 and the obj / best outputs are required");
-    if (max_rounds < 0) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": max_rounds >= 0 is required");
+    return SDPLRP_OK;
+}
+
+int32_t objective_check(sdplrp_handle *h, const char *name) {
     for (const LowRank &L : h->lr)
         if (L.gid == h->m) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": the objective has a low-rank part");
     if (h->obj_mat < 0) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": needs a sparse objective");
+    return SDPLRP_OK;
+}
+
+// hyperplanes on the host: the caller's G, or the counter-based normals (kept in Gh)
+const double *hyperplanes(const sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, std::vector<double> &Gh) {
+    if (G) return G;
+    const int r = h->r;
+    Gh.resize((size_t)K * r);
+    for (i64 k = 0; k < K; k++)
+        for (int c = 0; c < r; c++) Gh[(size_t)k * r + c] = hyperplane_normal(seed, k, c);
+    return Gh.data();
+}
+
+int32_t round_batches(sdplrp_handle *h, const char *name, int64_t K, const double *G, uint64_t seed, bool search, int64_t max_rounds,
+                      double *G_out, double *obj_round, double *obj, double *sum, int64_t *flips, int64_t *rounds, int64_t *best,
+                      double *best_x) {
+    SDP_CHECK(rounding_check(h, name, K, obj, best));
+    if (max_rounds < 0) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": max_rounds >= 0 is required");
+    SDP_CHECK(objective_check(h, name));
     CUDA_TRY(h, cudaSetDevice(h->device));
     const int r = h->r;
     const i64 n = h->n;
 
-    // hyperplanes on the host: the caller's, or the counter-based normals
     std::vector<double> Gh;
-    if (!G) {
-        Gh.resize((size_t)K * r);
-        for (i64 k = 0; k < K; k++)
-            for (int c = 0; c < r; c++) Gh[(size_t)k * r + c] = hyperplane_normal(seed, k, c);
-        G = Gh.data();
-    }
+    G = hyperplanes(h, K, G, seed, Gh);
     if (h->world > 1) {   // SPMD: every rank must round with the same K, the same hyperplanes and the same search
         unsigned long long cs = mix64((unsigned long long)K);
         if (search) cs = mix64(cs ^ (unsigned long long)(max_rounds + 1));
@@ -682,6 +1044,191 @@ int32_t round_batches(sdplrp_handle *h, const char *name, int64_t K, const doubl
     }
     return SDPLRP_OK;
 }
+
+// sweep buffers (first use after preprocessing)
+int32_t ensure_sweep_buffers(sdplrp_handle *h) {
+    RoundingState &s = h->rnd;
+    SDP_CHECK(ensure_segments(h));
+    if (s.sw_P) return SDPLRP_OK;
+    const i64 n = h->n;
+    if (n > 0x7fffffffLL) return fail(h, SDPLRP_ERR_ARG, "round_sweep: more than 2^31 - 1 vertices");
+    s.sw_ntiles = (n + kSwTile - 1) / kSwTile;
+    SDP_CHECK(dev_alloc(h, &s.sw_P, n * kSweepB));
+    SDP_CHECK(dev_alloc(h, &s.sw_delta, n * kSweepB));
+    SDP_CHECK(dev_alloc(h, &s.sw_order, n * kSweepB));
+    SDP_CHECK(dev_alloc(h, &s.sw_keys, 2 * n));
+    SDP_CHECK(dev_alloc(h, &s.sw_vals, n));
+    SDP_CHECK(dev_alloc(h, &s.sw_tiles, s.sw_ntiles * kSweepB * 5));
+    size_t bytes = 0;
+    CUDA_TRY(h, cub::DeviceRadixSort::SortPairs(nullptr, bytes, s.sw_keys, s.sw_keys + n, s.sw_vals, s.sw_order, (int)n, 0, 64,
+                                                h->stream));
+    SDP_CHECK(dev_alloc(h, &s.sw_cub, (i64)bytes));
+    s.sw_cub_bytes = bytes;
+    return SDPLRP_OK;
+}
+
+// one batch of nb <= 16 sweep candidates (hyperplanes dG): projection, sorts, delta pass, scan and selection (sel: nb x kSwSel),
+// then, when `words`, the words of the chosen vectors and, when esum != NULL, the evaluation pass.  prof (nb = 1): f(0..n).
+int32_t sweep_batch(sdplrp_handle *h, const double *dG, int nb, const double *w, double wlo, double whi, const double *csum,
+                    double *sel, double *prof, bool words, double *esum) {
+    RoundingState &s = h->rnd;
+    const i64 n = h->n, nrows = h->row_hi - h->row_lo, nt = s.sw_ntiles;
+    const int *iperm = h->relabeled ? h->iperm : nullptr, *perm = h->relabeled ? h->perm : nullptr;
+    const unsigned mask = (1u << nb) - 1u;
+    // 1. projections of the owned rows, all-gathered
+    k_round_sign<kSweepB, true><<<grid_for(std::max<i64>(nrows, 1), kSignTPB, 2 * kRedBlocks), kSignTPB, 0, h->stream>>>(
+        h->row_lo, nrows, h->r, h->R, dG, nb, nullptr, s.sw_P, nullptr, nullptr, nullptr);
+    KLAUNCH(h);
+    CUDA_TRY(h, cudaGetLastError());
+    SDP_CHECK(comm_gather_rowbytes(h, s.sw_P, kSweepB * sizeof(double)));
+    // 2. one stable radix sort per candidate of (key, input id): every rank sorts the whole vector
+    for (int k = 0; k < nb; k++) {
+        k_sw_keys<<<grid_for(n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(n, k, s.sw_P, perm, s.sw_keys, s.sw_vals);
+        KLAUNCH(h);
+        size_t bytes = s.sw_cub_bytes;
+        CUDA_TRY(h, cub::DeviceRadixSort::SortPairs(s.sw_cub, bytes, s.sw_keys, s.sw_keys + n, s.sw_vals, s.sw_order + (size_t)k * n,
+                                                    (int)n, 0, 64, h->stream));
+        h->launches += 4;
+    }
+    // 3. deltas of the owned rows, all-gathered
+    if (nrows > 0) {
+        k_sw_delta<<<grid_for(nrows, kLsTPB, 8 * kNumSM), kLsTPB, 0, h->stream>>>(h->row_lo, h->row_hi, h->full_ptr, h->full_idx, h->Cfull,
+                                                                                    s.sw_P, iperm, mask, s.sw_delta);
+        KLAUNCH(h);
+    }
+    if (s.s_hi > s.s_lo) {
+        k_sw_delta_seg<<<grid_for(s.s_hi - s.s_lo, 1, 8 * kNumSM), kLsTPB, 0, h->stream>>>(
+            s.s_lo, s.s_hi, s.seg_row, s.seg_start, h->full_ptr, h->full_idx, h->Cfull, s.sw_P, iperm, mask, s.seg_part);
+        KLAUNCH(h);
+        k_sw_delta_combine<<<grid_for(s.l_hi - s.l_lo, 128, 4 * kNumSM), 128, 0, h->stream>>>(s.l_lo, s.l_hi, s.long_rows, s.long_sptr,
+                                                                                              s.seg_part, s.sw_delta);
+        KLAUNCH(h);
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    SDP_CHECK(comm_gather_rowbytes(h, s.sw_delta, kSweepB * sizeof(double)));
+    // 4. three-phase scan and selection
+    double *tsum_d = s.sw_tiles, *tsum_w = tsum_d + nt * kSweepB, *tbest = tsum_w + nt * kSweepB;
+    k_sw_tile_sums<<<dim3((unsigned)nt, nb), kSwTPB, 0, h->stream>>>(n, nt, s.sw_order, s.sw_delta, w, tsum_d, tsum_w);
+    KLAUNCH(h);
+    k_sw_tile_scan<<<nb, kSwTPB, 0, h->stream>>>(nt, tsum_d, tsum_w);
+    KLAUNCH(h);
+    k_sw_scan<<<dim3((unsigned)nt, nb), kSwTPB, 0, h->stream>>>(n, nt, s.sw_order, s.sw_delta, w, tsum_d, tsum_w, csum, wlo, whi, prof,
+                                                               tbest);
+    KLAUNCH(h);
+    k_sw_select<<<nb, kSwTPB, 0, h->stream>>>(n, nt, tbest, s.sw_order, s.sw_P, iperm, sel);
+    KLAUNCH(h);
+    CUDA_TRY(h, cudaGetLastError());
+    if (!words) return SDPLRP_OK;
+    // 5. the chosen vectors as words, and their exact objective by the evaluation pass
+    if (nrows > 0) {
+        k_sw_words<<<grid_for(nrows, 256, kRedBlocks * 4), 256, 0, h->stream>>>(h->row_lo, h->row_hi, s.sw_P, iperm, sel, nb, s.words);
+        KLAUNCH(h);
+        CUDA_TRY(h, cudaGetLastError());
+    }
+    SDP_CHECK(comm_gather_rowbytes(h, s.words, sizeof(Word)));
+    if (esum) SDP_CHECK(eval_pass(h, nb, esum));
+    return SDPLRP_OK;
+}
+
+int32_t round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, const double *w, double wlo, double whi,
+                    double *G_out, double *obj, double *sum, double *wS, int64_t *thresh, int64_t *best, double *best_x,
+                    double *best_profile, int64_t *best_order) {
+    const char *name = "round_sweep";
+    SDP_CHECK(rounding_check(h, name, K, obj, best));
+    SDP_CHECK(objective_check(h, name));
+    if (std::isnan(wlo) || std::isnan(whi) || wlo > whi)
+        return fail(h, SDPLRP_ERR_ARG, "round_sweep: the window needs wlo <= whi (no NaN)");
+    const i64 n = h->n;
+    const int r = h->r;
+    if (w)
+        for (i64 i = 0; i < n; i++)
+            if (!(w[i] >= 0.0) || !std::isfinite(w[i]))
+                return fail(h, SDPLRP_ERR_ARG, "round_sweep: vertex weight " + std::to_string(i) + " is negative or not finite");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    std::vector<double> Gh;
+    G = hyperplanes(h, K, G, seed, Gh);
+    auto bits = [](double x) { unsigned long long b; memcpy(&b, &x, sizeof b); return b; };
+    if (h->world > 1) {   // SPMD: every rank must sweep with the same K, hyperplanes, weights and window
+        unsigned long long cs = mix64((unsigned long long)K ^ 0x5357454550ull);
+        for (i64 e = 0; e < K * r; e++) cs = mix64(cs ^ bits(G[e]));
+        cs = mix64(cs ^ bits(wlo));
+        cs = mix64(cs ^ bits(whi));
+        cs = mix64(cs ^ (w ? 1ull : 2ull));
+        if (w) for (i64 i = 0; i < n; i++) cs = mix64(cs ^ bits(w[i]));
+        SDP_CHECK(comm_check_same(h, cs, "hyperplanes (K, seed, G), weights or window"));
+    }
+
+    RoundingState &s = h->rnd;
+    SDP_CHECK(ensure_problem_buffers(h));
+    SDP_CHECK(ensure_sweep_buffers(h));
+    // sums: per batch 16 evaluation sums (all-reduced), then per batch + 1 (the recomputed best) 16 x kSwSel selections, sum of C
+    const i64 nbatch = (K + kSweepB - 1) / kSweepB;
+    const i64 sel_at = nbatch * kSweepB, csum_at = sel_at + (nbatch + 1) * kSweepB * kSwSel, sums_len = csum_at + 1;
+    SDP_CHECK(ensure(h, &s.G, &s.G_len, K * r));
+    SDP_CHECK(ensure(h, &s.sums, &s.sums_len, sums_len));
+    CUDA_TRY(h, cudaMemcpyAsync(s.G, G, (size_t)(K * r) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(s.sums, 0, (size_t)sums_len * sizeof(double), h->stream));
+    double *csum = s.sums + csum_at;
+    k_round_csum<<<kRedBlocks, 256, 0, h->stream>>>(h->nnzF, h->Cfull, h->partials, h->ticket, csum);   // replicated: same bits everywhere
+    KLAUNCH(h);
+    const double *wd = nullptr;
+    if (w) {
+        if (!s.sw_w) SDP_CHECK(dev_alloc(h, &s.sw_w, n));
+        SDP_CHECK(perm_upload(h, s.sw_w, w, 1, true));
+        wd = s.sw_w;
+    }
+    for (i64 bt = 0; bt < nbatch; bt++) {
+        const int nb = (int)std::min<i64>(kSweepB, K - bt * kSweepB);
+        SDP_CHECK(sweep_batch(h, s.G + (size_t)(bt * kSweepB) * r, nb, wd, wlo, whi, csum, s.sums + sel_at + bt * kSweepB * kSwSel,
+                              nullptr, true, s.sums + bt * kSweepB));
+    }
+    SDP_CHECK(comm_reduce_ptr(h, s.sums, (int)sel_at));
+    std::vector<double> hs((size_t)sums_len);
+    CUDA_TRY(h, cudaMemcpyAsync(hs.data(), s.sums, hs.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+
+    const double sumC = hs[(size_t)csum_at];
+    i64 kb = -1;
+    for (i64 k = 0; k < K; k++) {
+        const double *sl = hs.data() + sel_at + k * kSwSel;
+        const i64 t = (i64)sl[1];
+        const bool ok = t >= 0;
+        obj[k] = ok ? sumC - 2.0 * hs[(size_t)k] : INFINITY;
+        if (sum) sum[k] = ok ? (double)(n - 2 * t) : NAN;
+        if (wS) wS[k] = ok ? sl[2] : NAN;
+        if (thresh) thresh[k] = t;
+        if (ok && (kb < 0 || obj[k] < obj[kb])) kb = k;
+    }
+    if (kb < 0) return fail(h, SDPLRP_ERR_ARG, "round_sweep: no threshold of any candidate satisfies the weight window");
+    *best = kb + 1;
+    if (G_out) std::copy(G, G + (size_t)(K * r), G_out);
+    if (best_x || best_profile || best_order) {
+        // the best candidate alone (same FMA chain, sort, deltas and tiles: the same order, profile and vector)
+        if (best_profile) {
+            if (!s.sw_prof) SDP_CHECK(dev_alloc(h, &s.sw_prof, n + 1));
+        }
+        SDP_CHECK(sweep_batch(h, s.G + (size_t)kb * r, 1, wd, wlo, whi, csum, s.sums + sel_at + nbatch * kSweepB * kSwSel,
+                              best_profile ? s.sw_prof : nullptr, best_x != nullptr, nullptr));
+        if (best_x) {
+            k_round_expand<<<grid_for(n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(n, s.words, 0, s.x);
+            KLAUNCH(h);
+            CUDA_TRY(h, cudaGetLastError());
+            SDP_CHECK(perm_download(h, s.x, best_x, 1, true));
+        }
+        if (best_profile) {
+            CUDA_TRY(h, cudaMemcpyAsync(best_profile, s.sw_prof, (size_t)(n + 1) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        }
+        if (best_order) {
+            int64_t *ord = reinterpret_cast<int64_t *>(s.sw_keys);   // the sort is done: its key buffer holds the download
+            k_sw_order_out<<<grid_for(n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(n, s.sw_order, h->relabeled ? h->iperm : nullptr, ord);
+            KLAUNCH(h);
+            CUDA_TRY(h, cudaGetLastError());
+            CUDA_TRY(h, cudaMemcpyAsync(best_order, ord, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, h->stream));
+        }
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    }
+    return SDPLRP_OK;
+}
 }  // namespace
 
 void round_free(sdplrp_handle *h) {
@@ -693,6 +1240,10 @@ void round_free(sdplrp_handle *h) {
     s.G_len = s.sums_len = 0;
     s.e_lo = s.e_hi = s.nchunks = 0;
     s.n_seg = s.l_lo = s.l_hi = s.s_lo = s.s_hi = 0;
+    dev_free(&s.sw_P); dev_free(&s.sw_delta); dev_free(&s.sw_order); dev_free(&s.sw_keys); dev_free(&s.sw_vals); dev_free(&s.sw_cub);
+    dev_free(&s.sw_tiles); dev_free(&s.sw_w); dev_free(&s.sw_prof);
+    s.sw_cub_bytes = 0;
+    s.sw_ntiles = 0;
 }
 
 extern "C" int32_t sdplrp_round_hyperplane(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, double *G_out, double *obj,
@@ -707,4 +1258,11 @@ extern "C" int32_t sdplrp_round_local_search(sdplrp_handle *h, int64_t K, const 
     if (!h) return SDPLRP_ERR_ARG;
     return round_batches(h, "round_local_search", K, G, seed, max_rounds > 0 || rounds != nullptr, max_rounds, G_out, obj_round, obj,
                          sum, flips, rounds, best, best_x);
+}
+
+extern "C" int32_t sdplrp_round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed, const double *w, double wlo,
+                                      double whi, double *G_out, double *obj, double *sum, double *wS, int64_t *thresh, int64_t *best,
+                                      double *best_x, double *best_profile, int64_t *best_order) {
+    if (!h) return SDPLRP_ERR_ARG;
+    return round_sweep(h, K, G, seed, w, wlo, whi, G_out, obj, sum, wS, thresh, best, best_x, best_profile, best_order);
 }

@@ -269,6 +269,11 @@ class B200Engine:
         _lib.Handle.round_local_search."""
         return self.h.round_local_search(K, G, seed, max_rounds)
 
+    def round_sweep(self, K, G=None, seed=0, w=None, window=(-math.inf, math.inf)):
+        """K sweep roundings of the current R on the device, the best threshold of each projection R g_k inside a weight
+        window (sdplrp_round_sweep); see _lib.Handle.round_sweep."""
+        return self.h.round_sweep(K, G, seed, w, window)
+
     def close(self):
         self.h.close()
 
@@ -554,6 +559,31 @@ def hyperplane_rounding(ans, trials=64, seed=0, local_search_rounds=0):
     if local_search_rounds > 0:
         res.update(objs_rounded=out["obj_round"], flips=out["flips"], rounds=out["rounds"])
     return res
+
+
+def sweep_rounding(ans, trials=64, seed=0, weights=None, window=None, bisection=False):
+    """Sweep rounding of a solve: for each of `trials` random directions g_k (those of hyperplane_rounding with the same
+    seed), the vertices are sorted by <R_i, g_k> and every prefix S_t of that order is a candidate cut (x = -1 on S_t);
+    the one with the smallest <C, xx'> whose weight sum(weights[S_t]) lies in `window` is kept.  Everything runs on the
+    device.  `weights` defaults to 1 per vertex and `window` to no constraint; bisection=True sets the size window
+    [floor(n/2), ceil(n/2)] (exact bisections).  For a mu-balanced cut pass the degrees and (mu vol, (1 - mu) vol).
+    Returns {"x": the best +-1 vector (input vertex order), "obj", "objs", "sums", "trial" as hyperplane_rounding, and
+    "thresh" (per candidate, -1 where no prefix fits the window), "wS" (per candidate W(S_t)), "profile" (f(0..n) of the
+    best candidate) and "order" (its sweep order, 0-based input vertex ids)}."""
+    engine = ans["engine"]
+    if not hasattr(engine, "round_sweep"):
+        raise TypeError("sweep_rounding needs the GPU engine (the rounding passes run inside libsdplrp_b200.so)")
+    if bisection:
+        if weights is not None or window is not None:
+            raise ValueError("bisection=True sets the window on unit weights; pass either bisection or weights / window")
+        n = engine.n
+        window = (float(n // 2), float((n + 1) // 2))
+    if window is None:
+        window = (-math.inf, math.inf)
+    out = engine.round_sweep(int(trials), None, seed, weights, window)
+    k = out["best"]
+    return {"x": out["best_x"], "obj": float(out["obj"][k]), "objs": out["obj"], "sums": out["sum"], "trial": k,
+            "thresh": out["thresh"], "wS": out["wS"], "profile": out["best_profile"], "order": out["best_order"]}
 
 
 def _print_row(config, T, localiter, it, L, obj, sigma, gtol, ptol, gn, pn, gap, dual):
