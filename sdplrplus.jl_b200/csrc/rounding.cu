@@ -10,20 +10,19 @@
 // replicated full pattern, and the 2K partial sums (set bits, eval sums) are all-reduced once at the end.
 //
 // One-flip local search (sdplrp_round_local_search) runs on the same words between two evaluation passes.  Round t:
-//   want pass   k_ls_want (+ k_ls_want_seg / k_ls_want_combine for long rows): for every owned row flagged dirty,
+//   want pass   k_nbr_short / k_nbr_seg / k_nbr_combine<LsWant>: for every owned row flagged dirty,
 //               h_ik = sum_{j != i, C_ij != 0} C_ij x_jk for the 64 candidates, and bit k of want_i = (x_ik h_ik > 0).
-//               A row that is not dirty keeps its want word: it depends only on x_i and the x_j of its neighbours.
 //   flip pass   k_ls_flip (+ k_ls_flip_seg): flip_i = want_i & ~OR{want_j : j a neighbour with a higher priority}, and the
 //               per-candidate counts of wanting vertices.  The flipped vertices of a candidate are pairwise non-adjacent,
 //               so their gains add up and the objective falls by 4 sum |h_ik| every round.
 //   apply pass  k_ls_apply (+ k_ls_apply_seg): word_i ^= flip_i on every row, per-candidate flip counts over the owned
 //               rows, and a flipped row marks itself and its neighbours dirty (identical byte stores).
-// Rows with more than kLsLong nonzeros are cut into segments of kLsSeg nonzeros, one CTA each; the want sums of a long row
-// are combined over its segments in a fixed order.
+// Rows with more than kLsLong nonzeros are cut into segments of kLsSeg nonzeros, one CTA each; the want and delta sums of a
+// long row are combined over its segments in a fixed order.
 //
 // Sweep rounding (sdplrp_round_sweep) goes in batches of kSweepB = 16 candidates, one 128-byte row of projections per vertex:
-// projection pass (k_round_sign<16, true>) -> per candidate a stable radix sort of (key, input id) -> delta pass (k_sw_delta*,
-// the move deltas along each order) -> three-phase tile scan and selection (k_sw_tile_sums, k_sw_tile_scan, k_sw_scan,
+// projection pass (k_round_sign<16, true>) -> per candidate a stable radix sort of (key, input id) -> delta pass
+// (k_nbr_*<SwDelta>, the move deltas along each order) -> three-phase tile scan and selection (k_sw_tile_sums, k_sw_tile_scan, k_sw_scan,
 // k_sw_select) -> words of the chosen prefixes (k_sw_words) -> evaluation pass.  DESIGN.md §3f.
 // Nothing outside the rounding buffers (h->rnd) and the reduction scratch is written.
 #include <limits.h>
@@ -67,10 +66,16 @@ __device__ __forceinline__ void ballot_counts(Word w, int lane, unsigned (&cnt)[
     }
 }
 
-// the ballot counts of a thread as the 64 per-thread values of a grid reduction
-__device__ __forceinline__ void counts_to_values(const unsigned (&cnt)[2], int lane, double (&v)[kRoundB]) {
+// the ballot counts of every thread summed over the grid (fixed order) into out[k] for k < nb, stored or, when `add`, added
+__device__ __forceinline__ void counts_finalize(const unsigned (&cnt)[2], int lane, int nb, double *partials, unsigned *ticket,
+                                                double *out, bool add) {
+    double v[kRoundB];
 #pragma unroll
     for (int k = 0; k < kRoundB; k++) v[k] = lane == (k & 31) ? (double)cnt[k >> 5] : 0.0;
+    grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
+#pragma unroll
+        for (int k = 0; k < kRoundB; k++) if (k < nb) out[k] = add ? out[k] + s[k] : s[k];
+    });
 }
 
 // words[i] bit k = (<R_i, g_k> >= 0) for the owned rows; cnt[k] = number of set bits over them (k < 64).
@@ -126,14 +131,7 @@ __global__ void __launch_bounds__(kSignTPB) k_round_sign(i64 row_lo, i64 nrows, 
             ballot_counts(w, lane, cnt);
         }
     }
-    if constexpr (!PROJ) {
-        double v[kRoundB];
-        counts_to_values(cnt, lane, v);
-        grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
-#pragma unroll
-            for (int k = 0; k < kRoundB; k++) if (k < nb) cnt_out[k] = s[k];
-        });
-    }
+    if constexpr (!PROJ) counts_finalize(cnt, lane, nb, partials, ticket, cnt_out, false);
 }
 
 // first owned row of every chunk of kEvalChunk nonzeros (chunk c starts at nonzero e_lo + c * kEvalChunk)
@@ -226,70 +224,109 @@ __device__ __forceinline__ Word ls_want_word(Word wi, const double (&h)[kRoundB]
     return w & mask;
 }
 
-// want pass, rows with at most kLsLong nonzeros: one thread per dirty owned row, 64 register sums in pattern order
-__global__ void __launch_bounds__(kLsTPB) k_ls_want(i64 row_lo, i64 row_hi, const int *__restrict__ ptr, const int *__restrict__ idx,
-                                                   const double *__restrict__ val, const Word *__restrict__ words, Word mask,
-                                                   unsigned char *__restrict__ dirty, Word *__restrict__ want) {
+// nonzero e (column j) of row i is a neighbour in the sums and dirty marks: off the diagonal, with a nonzero value (read only
+// off the diagonal)
+template <class I>
+__device__ __forceinline__ bool is_neighbour(int j, I i, const double *__restrict__ val, int e) {
+    return j != i && val[e] != 0.0;
+}
+
+// segment s of long row i: nonzeros [e0, e1), at most kLsSeg of them
+__device__ __forceinline__ void seg_range(const int *__restrict__ seg_start, const int *__restrict__ ptr, i64 s, int i, int &e0,
+                                          int &e1) {
+    e0 = seg_start[s];
+    e1 = min(e0 + kLsSeg, ptr[i + 1]);
+}
+
+// ---- neighbour sums: acc_i[k] = sum over the neighbours j of row i of a term of (j, C_ij), for the want and delta passes --
+// Op supplies NB (sums per row), Row row(i) (per-row state), gather(j) (what the term reads of neighbour j),
+// add(row, gather(j), C_ij, acc), finish(i, acc) (writes row i's output) and kSegMinCTAs (resident CTAs per SM the
+// segment kernel is compiled for, 0: no bound).  With a gate (the local search's dirty flags), only the rows whose flag is
+// set are summed, and the flag is cleared when the row's output is written.  Rows with at most kLsLong nonzeros: one
+// thread per row, pattern order.  Long rows: one CTA per segment, thread-strided and block_sum into
+// part[s][k], then the segments of each row added in segment order.
+
+// want pass of the local search: h_ik = sum C_ij x_jk for the 64 candidates, on the dirty rows, and bit k of want_i =
+// (x_ik h_ik > 0).  A row that is not dirty keeps its want word: it depends only on x_i and the x_j of its neighbours.
+struct LsWant {
+    static constexpr int NB = kRoundB;
+    static constexpr int kSegMinCTAs = 0;
+    struct Row {};
+    const Word *words;
+    Word mask;
+    Word *want;
+    __device__ Row row(i64) const { return {}; }
+    __device__ Word gather(int j) const { return __ldg(words + j); }   // issued with idx / val, ahead of the neighbour test
+    __device__ void add(const Row &, Word wj, double v, double (&acc)[NB]) const { ls_accumulate(wj, v, acc); }
+    __device__ void finish(i64 i, const double (&acc)[NB]) const { want[i] = ls_want_word(__ldg(words + i), acc, mask); }
+};
+
+template <class Op>
+__global__ void __launch_bounds__(kLsTPB) k_nbr_short(i64 row_lo, i64 row_hi, const int *__restrict__ ptr, const int *__restrict__ idx,
+                                                     const double *__restrict__ val, const Op op, unsigned char *__restrict__ gate) {
     for (i64 i = row_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; i < row_hi; i += (i64)gridDim.x * blockDim.x) {
-        if (!dirty[i]) continue;
+        if (gate && !gate[i]) continue;
         const int a = ptr[i], b = ptr[i + 1];
         if (b - a > kLsLong) continue;
-        dirty[i] = 0;
-        double acc[kRoundB];
+        if (gate) gate[i] = 0;
+        const typename Op::Row row = op.row(i);
+        double acc[Op::NB];
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) acc[k] = 0.0;
+        for (int k = 0; k < Op::NB; k++) acc[k] = 0.0;
         for (int e = a; e < b; e++) {
             const int j = idx[e];
             const double v = val[e];
-            if (j == i || v == 0.0) continue;
-            ls_accumulate(words[j], v, acc);
+            const auto x = op.gather(j);
+            if (is_neighbour(j, i, val, e)) op.add(row, x, v, acc);
         }
-        want[i] = ls_want_word(words[i], acc, mask);
+        op.finish(i, acc);
     }
 }
 
-// want pass, long rows: one CTA per segment of a dirty owned row; part[s][k] = the segment's sums (fixed-order CTA sum)
-__global__ void __launch_bounds__(kLsTPB) k_ls_want_seg(i64 s_lo, i64 s_hi, const int *__restrict__ seg_row, const int *__restrict__ seg_start,
-                                                       const int *__restrict__ ptr, const int *__restrict__ idx,
-                                                       const double *__restrict__ val, const Word *__restrict__ words,
-                                                       const unsigned char *__restrict__ dirty, double *__restrict__ part) {
+template <class Op>
+__global__ void __launch_bounds__(kLsTPB, Op::kSegMinCTAs) k_nbr_seg(i64 s_lo, i64 s_hi, const int *__restrict__ seg_row,
+                                                                     const int *__restrict__ seg_start,
+                                                   const int *__restrict__ ptr, const int *__restrict__ idx,
+                                                   const double *__restrict__ val, const Op op, const unsigned char *__restrict__ gate,
+                                                   double *__restrict__ part) {
     for (i64 s = s_lo + blockIdx.x; s < s_hi; s += gridDim.x) {
         const int i = seg_row[s];
-        if (!dirty[i]) continue;   // the same for the whole CTA
-        const int e0 = seg_start[s], e1 = min(e0 + kLsSeg, ptr[i + 1]);
-        double acc[kRoundB];
+        if (gate && !gate[i]) continue;   // the same for the whole CTA
+        int e0, e1;
+        seg_range(seg_start, ptr, s, i, e0, e1);
+        const typename Op::Row row = op.row(i);
+        double acc[Op::NB];
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) acc[k] = 0.0;
+        for (int k = 0; k < Op::NB; k++) acc[k] = 0.0;
         for (int e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
             const int j = idx[e];
             const double v = val[e];
-            if (j == i || v == 0.0) continue;
-            ls_accumulate(words[j], v, acc);
+            const auto x = op.gather(j);
+            if (is_neighbour(j, i, val, e)) op.add(row, x, v, acc);
         }
-        block_sum<kRoundB>(acc);
+        block_sum<Op::NB>(acc);
         if (threadIdx.x == 0) {
 #pragma unroll
-            for (int k = 0; k < kRoundB; k++) part[(size_t)s * kRoundB + k] = acc[k];
+            for (int k = 0; k < Op::NB; k++) part[(size_t)s * Op::NB + k] = acc[k];
         }
     }
 }
 
-// want pass, long rows: the segment sums of every dirty owned long row added in segment order
-__global__ void k_ls_want_combine(i64 l_lo, i64 l_hi, const int *__restrict__ long_rows, const int *__restrict__ long_sptr,
-                                  const double *__restrict__ part, const Word *__restrict__ words, Word mask,
-                                  unsigned char *__restrict__ dirty, Word *__restrict__ want) {
+template <class Op>
+__global__ void k_nbr_combine(i64 l_lo, i64 l_hi, const int *__restrict__ long_rows, const int *__restrict__ long_sptr,
+                              const double *__restrict__ part, const Op op, unsigned char *__restrict__ gate) {
     for (i64 L = l_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; L < l_hi; L += (i64)gridDim.x * blockDim.x) {
         const int i = long_rows[L];
-        if (!dirty[i]) continue;
-        dirty[i] = 0;
-        double acc[kRoundB];
+        if (gate && !gate[i]) continue;
+        if (gate) gate[i] = 0;
+        double acc[Op::NB];
 #pragma unroll
-        for (int k = 0; k < kRoundB; k++) acc[k] = 0.0;
+        for (int k = 0; k < Op::NB; k++) acc[k] = 0.0;
         for (int s = long_sptr[L]; s < long_sptr[L + 1]; s++) {
 #pragma unroll
-            for (int k = 0; k < kRoundB; k++) acc[k] += part[(size_t)s * kRoundB + k];
+            for (int k = 0; k < Op::NB; k++) acc[k] += part[(size_t)s * Op::NB + k];
         }
-        want[i] = ls_want_word(words[i], acc, mask);
+        op.finish(i, acc);
     }
 }
 
@@ -315,19 +352,14 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_flip(i64 row_lo, i64 nrows, const
             for (int e = a; e < b && m != 0ull; e++) {
                 const int j = idx[e];
                 const Word wj = want[j] & m;
-                if (wj == 0ull || j == i || val[e] == 0.0) continue;
+                if (wj == 0ull || !is_neighbour(j, i, val, e)) continue;
                 const Word kj = ls_key(iperm, j, salt, rj);
                 if (ls_beats(kj, rj, ki, ri)) m &= ~wj;
             }
         }
         flip[i] = m;
     }
-    double v[kRoundB];
-    counts_to_values(cnt, lane, v);
-    grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
-#pragma unroll
-        for (int k = 0; k < kRoundB; k++) if (k < nb) cnt_out[k] = s[k];
-    });
+    counts_finalize(cnt, lane, nb, partials, ticket, cnt_out, false);
 }
 
 // flip pass, long rows: one CTA per segment of an owned long row that wants to flip; clears the bits a beating neighbour
@@ -342,11 +374,12 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_flip_seg(i64 s_lo, i64 s_hi, cons
         if (wi == 0ull) continue;
         Word ri, rj, blocked = 0ull;
         const Word ki = ls_key(iperm, i, salt, ri);
-        const int e0 = seg_start[s], e1 = min(e0 + kLsSeg, ptr[i + 1]);
+        int e0, e1;
+        seg_range(seg_start, ptr, s, i, e0, e1);
         for (int e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
             const int j = idx[e];
             const Word wj = want[j] & wi;
-            if (wj == 0ull || j == i || val[e] == 0.0) continue;
+            if (wj == 0ull || !is_neighbour(j, i, val, e)) continue;
             const Word kj = ls_key(iperm, j, salt, rj);
             if (ls_beats(kj, rj, ki, ri)) blocked |= wj;
         }
@@ -375,15 +408,10 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_apply(i64 n, i64 row_lo, i64 row_
         if (b - a > kLsLong) continue;
         for (int e = a; e < b; e++) {
             const int j = idx[e];
-            if (j != i && val[e] != 0.0) dirty[j] = 1;
+            if (is_neighbour(j, i, val, e)) dirty[j] = 1;
         }
     }
-    double v[kRoundB];
-    counts_to_values(cnt, lane, v);
-    grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
-#pragma unroll
-        for (int k = 0; k < kRoundB; k++) if (k < nb) flips_acc[k] += s[k];
-    });
+    counts_finalize(cnt, lane, nb, partials, ticket, flips_acc, true);
 }
 
 // apply pass, long rows: one CTA per segment of a flipped row marks the segment's neighbours dirty
@@ -394,10 +422,11 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_apply_seg(i64 nseg, const int *__
     for (i64 s = blockIdx.x; s < nseg; s += gridDim.x) {
         const int i = seg_row[s];
         if (flip[i] == 0ull) continue;
-        const int e0 = seg_start[s], e1 = min(e0 + kLsSeg, ptr[i + 1]);
+        int e0, e1;
+        seg_range(seg_start, ptr, s, i, e0, e1);
         for (int e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
             const int j = idx[e];
-            if (j != i && val[e] != 0.0) dirty[j] = 1;
+            if (is_neighbour(j, i, val, e)) dirty[j] = 1;
         }
     }
 }
@@ -411,12 +440,7 @@ __global__ void __launch_bounds__(kLsTPB) k_ls_count(i64 row_lo, i64 nrows, cons
         const bool valid = base + threadIdx.x < nrows;
         ballot_counts(valid ? words[row_lo + base + threadIdx.x] : 0ull, lane, cnt);
     }
-    double v[kRoundB];
-    counts_to_values(cnt, lane, v);
-    grid_sum_finalize<kRoundB>(v, partials, ticket, [&](double (&s)[kRoundB]) {
-#pragma unroll
-        for (int k = 0; k < kRoundB; k++) if (k < nb) cnt_out[k] = s[k];
-    });
+    counts_finalize(cnt, lane, nb, partials, ticket, cnt_out, false);
 }
 
 // ---- sweep rounding --------------------------------------------------------------------------------------------------
@@ -455,74 +479,32 @@ __global__ void k_sw_keys(i64 n, int k, const double *__restrict__ P, const int 
     }
 }
 
-// delta pass, rows with at most kLsLong nonzeros: one thread per owned row, delta[v][k] = -4 (sum_after C_vj - sum_before C_vj)
-__global__ void __launch_bounds__(kLsTPB) k_sw_delta(i64 row_lo, i64 row_hi, const int *__restrict__ ptr, const int *__restrict__ idx,
-                                                    const double *__restrict__ val, const double *__restrict__ P,
-                                                    const int *__restrict__ iperm, unsigned mask, double *__restrict__ delta) {
-    for (i64 i = row_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; i < row_hi; i += (i64)gridDim.x * blockDim.x) {
-        const int a = ptr[i], b = ptr[i + 1];
-        if (b - a > kLsLong) continue;
-        double pv[kSweepB], acc[kSweepB];
-        sw_load_row(P, i, pv);
-        const int rv = sw_ref(iperm, i);
-#pragma unroll
-        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
-        for (int e = a; e < b; e++) {
-            const int j = idx[e];
-            const double v = val[e];
-            if (j == i || v == 0.0) continue;
-            sw_accumulate(P, iperm, j, v, pv, rv, mask, acc);
-        }
+// delta pass of the sweep: delta[v][k] = -4 (sum_after C_vj - sum_before C_vj) along candidate k's order, on every row
+struct SwDelta {
+    static constexpr int NB = kSweepB;
+    static constexpr int kSegMinCTAs = 5;   // at most 96 registers: the 128-byte row gathers of hub rows want the occupancy
+    struct Row {
+        double p[kSweepB];
+        int ref;
+    };
+    const double *P;
+    const int *iperm;
+    unsigned mask;
+    double *delta;
+    __device__ Row row(i64 i) const {
+        Row r;
+        sw_load_row(P, i, r.p);
+        r.ref = sw_ref(iperm, i);
+        return r;
+    }
+    __device__ int gather(int j) const { return j; }   // the row of P is read in add, after the neighbour test
+    __device__ void add(const Row &r, int j, double v, double (&acc)[NB]) const { sw_accumulate(P, iperm, j, v, r.p, r.ref, mask, acc); }
+    __device__ void finish(i64 i, const double (&acc)[NB]) const {
         double2 *out = reinterpret_cast<double2 *>(delta + (size_t)i * kSweepB);
 #pragma unroll
         for (int k = 0; k < kSweepB; k += 2) out[k / 2] = make_double2(-4.0 * acc[k], -4.0 * acc[k + 1]);
     }
-}
-
-// delta pass, long rows: one CTA per segment of an owned long row; part[s][k] = the segment's signed sums (fixed-order CTA sum)
-__global__ void __launch_bounds__(kLsTPB) k_sw_delta_seg(i64 s_lo, i64 s_hi, const int *__restrict__ seg_row,
-                                                        const int *__restrict__ seg_start, const int *__restrict__ ptr,
-                                                        const int *__restrict__ idx, const double *__restrict__ val,
-                                                        const double *__restrict__ P, const int *__restrict__ iperm, unsigned mask,
-                                                        double *__restrict__ part) {
-    for (i64 s = s_lo + blockIdx.x; s < s_hi; s += gridDim.x) {
-        const int i = seg_row[s];
-        const int e0 = seg_start[s], e1 = min(e0 + kLsSeg, ptr[i + 1]);
-        double pv[kSweepB], acc[kSweepB];
-        sw_load_row(P, i, pv);
-        const int rv = sw_ref(iperm, i);
-#pragma unroll
-        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
-        for (int e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
-            const int j = idx[e];
-            const double v = val[e];
-            if (j == i || v == 0.0) continue;
-            sw_accumulate(P, iperm, j, v, pv, rv, mask, acc);
-        }
-        block_sum<kSweepB>(acc);
-        if (threadIdx.x == 0) {
-#pragma unroll
-            for (int k = 0; k < kSweepB; k++) part[(size_t)s * kSweepB + k] = acc[k];
-        }
-    }
-}
-
-// delta pass, long rows: the segment sums of every owned long row added in segment order
-__global__ void k_sw_delta_combine(i64 l_lo, i64 l_hi, const int *__restrict__ long_rows, const int *__restrict__ long_sptr,
-                                   const double *__restrict__ part, double *__restrict__ delta) {
-    for (i64 L = l_lo + blockIdx.x * (i64)blockDim.x + threadIdx.x; L < l_hi; L += (i64)gridDim.x * blockDim.x) {
-        double acc[kSweepB];
-#pragma unroll
-        for (int k = 0; k < kSweepB; k++) acc[k] = 0.0;
-        for (int s = long_sptr[L]; s < long_sptr[L + 1]; s++) {
-#pragma unroll
-            for (int k = 0; k < kSweepB; k++) acc[k] += part[(size_t)s * kSweepB + k];
-        }
-        double *out = delta + (size_t)long_rows[L] * kSweepB;
-#pragma unroll
-        for (int k = 0; k < kSweepB; k++) out[k] = -4.0 * acc[k];
-    }
-}
+};
 
 // exclusive prefix of (a, b) over the threads of the CTA in thread order (shuffle scans: the same bits every run)
 __device__ __forceinline__ void sw_block_exscan(double &a, double &b) {
@@ -828,6 +810,29 @@ int32_t ensure_segments(sdplrp_handle *h) {
     return SDPLRP_OK;
 }
 
+// the neighbour sums of op over the owned rows (kernels above), gated by `gate` unless it is NULL; the long rows' segment
+// sums go through seg_part
+template <class Op>
+int32_t neighbour_sums(sdplrp_handle *h, const Op &op, unsigned char *gate) {
+    RoundingState &s = h->rnd;
+    const i64 nrows = h->row_hi - h->row_lo;
+    if (nrows > 0) {
+        k_nbr_short<Op><<<grid_for(nrows, kLsTPB, 8 * kNumSM), kLsTPB, 0, h->stream>>>(h->row_lo, h->row_hi, h->full_ptr, h->full_idx,
+                                                                                        h->Cfull, op, gate);
+        KLAUNCH(h);
+    }
+    if (s.s_hi > s.s_lo) {
+        k_nbr_seg<Op><<<grid_for(s.s_hi - s.s_lo, 1, 8 * kNumSM), kLsTPB, 0, h->stream>>>(
+            s.s_lo, s.s_hi, s.seg_row, s.seg_start, h->full_ptr, h->full_idx, h->Cfull, op, gate, s.seg_part);
+        KLAUNCH(h);
+        k_nbr_combine<Op><<<grid_for(s.l_hi - s.l_lo, 128, 4 * kNumSM), 128, 0, h->stream>>>(s.l_lo, s.l_hi, s.long_rows, s.long_sptr,
+                                                                                             s.seg_part, op, gate);
+        KLAUNCH(h);
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    return SDPLRP_OK;
+}
+
 // local-search buffers (first use after preprocessing): the segments, want / flip / best words and dirty flags (n each)
 int32_t ensure_search_buffers(sdplrp_handle *h) {
     RoundingState &s = h->rnd;
@@ -855,19 +860,7 @@ int32_t local_search(sdplrp_handle *h, int nb, i64 max_rounds, double *wcnt, dou
     CUDA_TRY(h, cudaMemsetAsync(s.dirty, 1, (size_t)n, h->stream));
     for (i64 t = 0;; t++) {
         const Word salt = mix64(0xD1B54A32D192ED03ull * (Word)(t + 1));
-        if (nrows > 0) {
-            k_ls_want<<<grid_for(nrows, kLsTPB, 8 * kNumSM), kLsTPB, 0, h->stream>>>(h->row_lo, h->row_hi, h->full_ptr, h->full_idx,
-                                                                                       h->Cfull, s.words, mask, s.dirty, s.want);
-            KLAUNCH(h);
-        }
-        if (s.s_hi > s.s_lo) {
-            k_ls_want_seg<<<grid_for(s.s_hi - s.s_lo, 1, 8 * kNumSM), kLsTPB, 0, h->stream>>>(
-                s.s_lo, s.s_hi, s.seg_row, s.seg_start, h->full_ptr, h->full_idx, h->Cfull, s.words, s.dirty, s.seg_part);
-            KLAUNCH(h);
-            k_ls_want_combine<<<grid_for(s.l_hi - s.l_lo, 128, 4 * kNumSM), 128, 0, h->stream>>>(
-                s.l_lo, s.l_hi, s.long_rows, s.long_sptr, s.seg_part, s.words, mask, s.dirty, s.want);
-            KLAUNCH(h);
-        }
+        SDP_CHECK(neighbour_sums(h, LsWant{s.words, mask, s.want}, s.dirty));
         SDP_CHECK(comm_gather_rowbytes(h, s.want, sizeof(Word)));
         k_ls_flip<<<grid_for(std::max<i64>(nrows, 1), kLsTPB, 2 * kRedBlocks), kLsTPB, 0, h->stream>>>(
             h->row_lo, nrows, h->full_ptr, h->full_idx, h->Cfull, iperm, salt, s.want, s.flip, nb, h->partials, h->ticket, wcnt);
@@ -906,8 +899,6 @@ int32_t local_search(sdplrp_handle *h, int nb, i64 max_rounds, double *wcnt, dou
 // per batch of 64 candidates, a block of sums: set bits, final eval sums, first eval sums (before the search), flips
 constexpr int kSumBlock = 4 * kRoundB;
 
-// K candidates in batches of 64: sign pass, all-gather of the words, evaluation pass and, when `search`, the one-flip
-// descent and a second evaluation pass.  sdplrp_round_hyperplane is the case without search.
 // the checks every rounding entry point makes before it touches the device
 int32_t rounding_check(sdplrp_handle *h, const char *name, int64_t K, const void *obj, const void *best) {
     if (!h->preprocessed) return fail(h, SDPLRP_ERR_STATE, "call sdplrp_preprocess first");
@@ -933,38 +924,65 @@ const double *hyperplanes(const sdplrp_handle *h, int64_t K, const double *G, ui
     return Gh.data();
 }
 
+Word double_bits(double x) {
+    Word b;
+    memcpy(&b, &x, sizeof b);
+    return b;
+}
+
+// The device half of every rounding call, after its argument checks.  G becomes the hyperplanes (the caller's, or the
+// seeded normals kept in Gh).  Several GPUs: every rank must round the same call, so a checksum of K ^ salt, the
+// hyperplanes, `extra` and the bits of tail[0..ntail) is compared across ranks ("what" names them in the error).  Then the
+// problem buffers, G on the device, sums_len zeroed sums and the sum of C at sums[csum_at] (replicated: same bits everywhere).
+int32_t round_setup(sdplrp_handle *h, int64_t K, const double *&G, uint64_t seed, std::vector<double> &Gh, Word salt,
+                    std::initializer_list<Word> extra, const double *tail, i64 ntail, const char *what, i64 sums_len, i64 csum_at) {
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    const i64 len = K * h->r;
+    G = hyperplanes(h, K, G, seed, Gh);
+    if (h->world > 1) {
+        Word cs = mix64((Word)K ^ salt);
+        for (i64 e = 0; e < len; e++) cs = mix64(cs ^ double_bits(G[e]));
+        for (Word x : extra) cs = mix64(cs ^ x);
+        for (i64 e = 0; e < ntail; e++) cs = mix64(cs ^ double_bits(tail[e]));
+        SDP_CHECK(comm_check_same(h, cs, what));
+    }
+    RoundingState &s = h->rnd;
+    SDP_CHECK(ensure_problem_buffers(h));
+    SDP_CHECK(ensure(h, &s.G, &s.G_len, len));
+    SDP_CHECK(ensure(h, &s.sums, &s.sums_len, sums_len));
+    CUDA_TRY(h, cudaMemcpyAsync(s.G, G, (size_t)len * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(s.sums, 0, (size_t)sums_len * sizeof(double), h->stream));
+    k_round_csum<<<kRedBlocks, 256, 0, h->stream>>>(h->nnzF, h->Cfull, h->partials, h->ticket, s.sums + csum_at);
+    KLAUNCH(h);
+    return SDPLRP_OK;
+}
+
+// best_x (input order) = +1 / -1 from bit b of the words
+int32_t download_signs(sdplrp_handle *h, const Word *words, int b, double *best_x) {
+    k_round_expand<<<grid_for(h->n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(h->n, words, b, h->rnd.x);
+    KLAUNCH(h);
+    CUDA_TRY(h, cudaGetLastError());
+    return perm_download(h, h->rnd.x, best_x, 1, true);
+}
+
+// K candidates in batches of 64: sign pass, all-gather of the words, evaluation pass and, when `search`, the one-flip
+// descent and a second evaluation pass.  sdplrp_round_hyperplane is the case without search.
 int32_t round_batches(sdplrp_handle *h, const char *name, int64_t K, const double *G, uint64_t seed, bool search, int64_t max_rounds,
                       double *G_out, double *obj_round, double *obj, double *sum, int64_t *flips, int64_t *rounds, int64_t *best,
                       double *best_x) {
     SDP_CHECK(rounding_check(h, name, K, obj, best));
     if (max_rounds < 0) return fail(h, SDPLRP_ERR_ARG, std::string(name) + ": max_rounds >= 0 is required");
     SDP_CHECK(objective_check(h, name));
-    CUDA_TRY(h, cudaSetDevice(h->device));
     const int r = h->r;
     const i64 n = h->n;
-
-    std::vector<double> Gh;
-    G = hyperplanes(h, K, G, seed, Gh);
-    if (h->world > 1) {   // SPMD: every rank must round with the same K, the same hyperplanes and the same search
-        unsigned long long cs = mix64((unsigned long long)K);
-        if (search) cs = mix64(cs ^ (unsigned long long)(max_rounds + 1));
-        const unsigned long long *bits = reinterpret_cast<const unsigned long long *>(G);
-        for (i64 e = 0; e < K * r; e++) cs = mix64(cs ^ bits[e]);
-        SDP_CHECK(comm_check_same(h, cs, "hyperplanes (K, seed, G) or max_rounds"));
-    }
-
-    RoundingState &s = h->rnd;
-    SDP_CHECK(ensure_problem_buffers(h));
-    if (search) SDP_CHECK(ensure_search_buffers(h));
     const i64 nbatch = (K + kRoundB - 1) / kRoundB;
     const i64 csum_at = nbatch * kSumBlock, sums_len = csum_at + 1 + kRoundB;   // + sum of C, + want counts of a round
-    SDP_CHECK(ensure(h, &s.G, &s.G_len, K * r));
-    SDP_CHECK(ensure(h, &s.sums, &s.sums_len, sums_len));
-    CUDA_TRY(h, cudaMemcpyAsync(s.G, G, (size_t)(K * r) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemsetAsync(s.sums, 0, (size_t)sums_len * sizeof(double), h->stream));
+    std::vector<double> Gh;
+    SDP_CHECK(round_setup(h, K, G, seed, Gh, 0, {search ? (Word)(max_rounds + 1) : 0}, nullptr, 0,
+                          "hyperplanes (K, seed, G) or max_rounds", sums_len, csum_at));
+    RoundingState &s = h->rnd;
+    if (search) SDP_CHECK(ensure_search_buffers(h));
     double *csum = s.sums + csum_at, *wcnt = csum + 1;
-    k_round_csum<<<kRedBlocks, 256, 0, h->stream>>>(h->nnzF, h->Cfull, h->partials, h->ticket, csum);   // replicated: same bits everywhere
-    KLAUNCH(h);
     double sumC = 0.0;
     if (search) {
         CUDA_TRY(h, cudaMemcpyAsync(&sumC, csum, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -1037,10 +1055,7 @@ int32_t round_batches(sdplrp_handle *h, const char *name, int64_t K, const doubl
             SDP_CHECK(sign_pass(h, s.G + (size_t)(bt * kRoundB) * r, nb, s.sums + bt * kSumBlock));
             SDP_CHECK(comm_gather_rowbytes(h, s.words, sizeof(Word)));
         }
-        k_round_expand<<<grid_for(n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(n, bw, (int)(kb - bt * kRoundB), s.x);
-        KLAUNCH(h);
-        CUDA_TRY(h, cudaGetLastError());
-        SDP_CHECK(perm_download(h, s.x, best_x, 1, true));
+        SDP_CHECK(download_signs(h, bw, (int)(kb - bt * kRoundB), best_x));
     }
     return SDPLRP_OK;
 }
@@ -1091,20 +1106,7 @@ int32_t sweep_batch(sdplrp_handle *h, const double *dG, int nb, const double *w,
         h->launches += 4;
     }
     // 3. deltas of the owned rows, all-gathered
-    if (nrows > 0) {
-        k_sw_delta<<<grid_for(nrows, kLsTPB, 8 * kNumSM), kLsTPB, 0, h->stream>>>(h->row_lo, h->row_hi, h->full_ptr, h->full_idx, h->Cfull,
-                                                                                    s.sw_P, iperm, mask, s.sw_delta);
-        KLAUNCH(h);
-    }
-    if (s.s_hi > s.s_lo) {
-        k_sw_delta_seg<<<grid_for(s.s_hi - s.s_lo, 1, 8 * kNumSM), kLsTPB, 0, h->stream>>>(
-            s.s_lo, s.s_hi, s.seg_row, s.seg_start, h->full_ptr, h->full_idx, h->Cfull, s.sw_P, iperm, mask, s.seg_part);
-        KLAUNCH(h);
-        k_sw_delta_combine<<<grid_for(s.l_hi - s.l_lo, 128, 4 * kNumSM), 128, 0, h->stream>>>(s.l_lo, s.l_hi, s.long_rows, s.long_sptr,
-                                                                                              s.seg_part, s.sw_delta);
-        KLAUNCH(h);
-    }
-    CUDA_TRY(h, cudaGetLastError());
+    SDP_CHECK(neighbour_sums(h, SwDelta{s.sw_P, iperm, mask, s.sw_delta}, nullptr));
     SDP_CHECK(comm_gather_rowbytes(h, s.sw_delta, kSweepB * sizeof(double)));
     // 4. three-phase scan and selection
     double *tsum_d = s.sw_tiles, *tsum_w = tsum_d + nt * kSweepB, *tbest = tsum_w + nt * kSweepB;
@@ -1144,33 +1146,15 @@ int32_t round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed,
         for (i64 i = 0; i < n; i++)
             if (!(w[i] >= 0.0) || !std::isfinite(w[i]))
                 return fail(h, SDPLRP_ERR_ARG, "round_sweep: vertex weight " + std::to_string(i) + " is negative or not finite");
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    std::vector<double> Gh;
-    G = hyperplanes(h, K, G, seed, Gh);
-    auto bits = [](double x) { unsigned long long b; memcpy(&b, &x, sizeof b); return b; };
-    if (h->world > 1) {   // SPMD: every rank must sweep with the same K, hyperplanes, weights and window
-        unsigned long long cs = mix64((unsigned long long)K ^ 0x5357454550ull);
-        for (i64 e = 0; e < K * r; e++) cs = mix64(cs ^ bits(G[e]));
-        cs = mix64(cs ^ bits(wlo));
-        cs = mix64(cs ^ bits(whi));
-        cs = mix64(cs ^ (w ? 1ull : 2ull));
-        if (w) for (i64 i = 0; i < n; i++) cs = mix64(cs ^ bits(w[i]));
-        SDP_CHECK(comm_check_same(h, cs, "hyperplanes (K, seed, G), weights or window"));
-    }
-
-    RoundingState &s = h->rnd;
-    SDP_CHECK(ensure_problem_buffers(h));
-    SDP_CHECK(ensure_sweep_buffers(h));
     // sums: per batch 16 evaluation sums (all-reduced), then per batch + 1 (the recomputed best) 16 x kSwSel selections, sum of C
     const i64 nbatch = (K + kSweepB - 1) / kSweepB;
     const i64 sel_at = nbatch * kSweepB, csum_at = sel_at + (nbatch + 1) * kSweepB * kSwSel, sums_len = csum_at + 1;
-    SDP_CHECK(ensure(h, &s.G, &s.G_len, K * r));
-    SDP_CHECK(ensure(h, &s.sums, &s.sums_len, sums_len));
-    CUDA_TRY(h, cudaMemcpyAsync(s.G, G, (size_t)(K * r) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemsetAsync(s.sums, 0, (size_t)sums_len * sizeof(double), h->stream));
+    std::vector<double> Gh;
+    SDP_CHECK(round_setup(h, K, G, seed, Gh, 0x5357454550ull, {double_bits(wlo), double_bits(whi), w ? 1ull : 2ull}, w, w ? n : 0,
+                          "hyperplanes (K, seed, G), weights or window", sums_len, csum_at));
+    RoundingState &s = h->rnd;
+    SDP_CHECK(ensure_sweep_buffers(h));
     double *csum = s.sums + csum_at;
-    k_round_csum<<<kRedBlocks, 256, 0, h->stream>>>(h->nnzF, h->Cfull, h->partials, h->ticket, csum);   // replicated: same bits everywhere
-    KLAUNCH(h);
     const double *wd = nullptr;
     if (w) {
         if (!s.sw_w) SDP_CHECK(dev_alloc(h, &s.sw_w, n));
@@ -1209,12 +1193,7 @@ int32_t round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed,
         }
         SDP_CHECK(sweep_batch(h, s.G + (size_t)kb * r, 1, wd, wlo, whi, csum, s.sums + sel_at + nbatch * kSweepB * kSwSel,
                               best_profile ? s.sw_prof : nullptr, best_x != nullptr, nullptr));
-        if (best_x) {
-            k_round_expand<<<grid_for(n, 256, kRedBlocks * 4), 256, 0, h->stream>>>(n, s.words, 0, s.x);
-            KLAUNCH(h);
-            CUDA_TRY(h, cudaGetLastError());
-            SDP_CHECK(perm_download(h, s.x, best_x, 1, true));
-        }
+        if (best_x) SDP_CHECK(download_signs(h, s.words, 0, best_x));
         if (best_profile) {
             CUDA_TRY(h, cudaMemcpyAsync(best_profile, s.sw_prof, (size_t)(n + 1) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         }
@@ -1233,8 +1212,7 @@ int32_t round_sweep(sdplrp_handle *h, int64_t K, const double *G, uint64_t seed,
 
 void round_free(sdplrp_handle *h) {
     RoundingState &s = h->rnd;
-    if (s.words) { cudaFree(s.words); s.words = nullptr; }
-    dev_free(&s.x); dev_free(&s.chunk_row); dev_free(&s.G); dev_free(&s.sums);
+    dev_free(&s.words); dev_free(&s.x); dev_free(&s.chunk_row); dev_free(&s.G); dev_free(&s.sums);
     dev_free(&s.want); dev_free(&s.flip); dev_free(&s.best_words); dev_free(&s.dirty);
     dev_free(&s.long_rows); dev_free(&s.long_sptr); dev_free(&s.seg_row); dev_free(&s.seg_start); dev_free(&s.seg_part);
     s.G_len = s.sums_len = 0;

@@ -2,92 +2,14 @@
 restatement of the same algorithm: start vectors, every round's priorities and flips, the objectives, sums, flip and round
 counts, the best candidate and its vector (exact where the gains are exactly representable), and the one-flip local
 optimality of the results for real weights."""
-import itertools
-
 import numpy as np
 import pytest
 import scipy.sparse as sps
 
 from helpers import COMBOS, families, g1_graph, make_case
+from rounding_reference import check_against_reference, engine_with_R, numpy_local_search, offdiag, start_vectors
 
 pytestmark = pytest.mark.gpu
-
-M64 = (1 << 64) - 1
-
-
-def mix64(x):
-    """splitmix64 finalizer on a uint64 array (wrap-around arithmetic)"""
-    x = np.asarray(x, dtype=np.uint64)
-    with np.errstate(over="ignore"):
-        x = x + np.uint64(0x9E3779B97F4A7C15)
-        x = (x ^ (x >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
-        x = (x ^ (x >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
-    return x ^ (x >> np.uint64(31))
-
-
-def priorities(n, t):
-    """key(i, t) = mix64(i ^ mix64(0xD1B54A32D192ED03 * (t + 1))) for i = 0..n-1"""
-    salt = mix64(np.array([(0xD1B54A32D192ED03 * (t + 1)) & M64], dtype=np.uint64))[0]
-    return mix64(np.arange(n, dtype=np.uint64) ^ salt)
-
-
-def offdiag(C):
-    A = sps.csr_matrix(C, dtype=np.float64).copy()
-    A.setdiag(0.0)
-    A.eliminate_zeros()
-    return A
-
-
-def numpy_local_search(C, X0, max_rounds):
-    """Parallel one-flip descent of every column of X0: per round, h = (C - diag C) x, i wants to flip iff x_i h_i > 0, and
-    flips iff no neighbour with a higher priority also wants to.  Returns X, obj, sum, flips, rounds (the last round that
-    flipped the candidate, 0 if none, -1 if it still wanted to flip after max_rounds rounds)."""
-    A = offdiag(C)
-    n, K = X0.shape
-    coo = A.tocoo()
-    rows, cols = coo.row.astype(np.int64), coo.col.astype(np.int64)
-    X = X0.copy()
-    flips, rounds = np.zeros(K, np.int64), np.zeros(K, np.int64)
-    for t in itertools.count():
-        W = X * (A @ X) > 0
-        cnt = W.sum(axis=0)
-        if not cnt.any():
-            break
-        if t == max_rounds:
-            rounds[cnt > 0] = -1
-            break
-        key = priorities(n, t)
-        F = W.copy()
-        for k in np.flatnonzero(cnt):
-            w = W[:, k]
-            sel = w[rows] & w[cols]   # both ends want to flip
-            ri, cj = rows[sel], cols[sel]
-            beats = (key[cj] > key[ri]) | ((key[cj] == key[ri]) & (cj < ri))   # neighbour j beats i
-            F[ri[beats], k] = False
-        X[F] *= -1.0
-        flips += F.sum(axis=0)
-        rounds[cnt > 0] = t + 1
-    obj = np.einsum("ik,ik->k", X, sps.csr_matrix(C) @ X)
-    return X, obj, X.sum(axis=0), flips, rounds
-
-
-def start_vectors(R, G):
-    return np.where(R @ G.T >= 0, 1.0, -1.0)
-
-
-def check_against_reference(res, C, X0, max_rounds):
-    X, obj, tot, flips, rounds = numpy_local_search(C, X0, max_rounds)
-    obj0 = np.einsum("ik,ik->k", X0, sps.csr_matrix(C) @ X0)
-    np.testing.assert_array_equal(res["obj_round"], obj0)
-    np.testing.assert_array_equal(res["obj"], obj)
-    np.testing.assert_array_equal(res["sum"], tot)
-    np.testing.assert_array_equal(res["flips"], flips)
-    np.testing.assert_array_equal(res["rounds"], rounds)
-    b = res["best"]
-    assert b == int(np.argmin(obj))
-    np.testing.assert_array_equal(res["best_x"], X[:, b])
-    return X
-
 
 def check_local_optimum(res, C, rtol=0.0):
     """obj <= obj_round, obj of best_x, and x_i h_i <= 0 on best_x (every candidate with rounds >= 0 is checked through
@@ -101,12 +23,6 @@ def check_local_optimum(res, C, rtol=0.0):
     if res["rounds"][res["best"]] >= 0:
         h = offdiag(C) @ x
         assert np.all(x * h <= rtol * (abs(offdiag(C)) @ np.ones_like(x) + 1.0))
-
-
-def engine_with_R(sp, gpu_handle_factory, config, C, As, bs, R):
-    eng = sp.B200Engine(sp.SDPData(C, As, bs), handle=gpu_handle_factory(config))
-    eng.init_vars(R.shape[1], R, np.zeros(C.shape[0]), 2.0, 4)
-    return eng
 
 
 def graphs(sp):
@@ -317,21 +233,3 @@ def test_powerlaw_million_vertices(sp, gpu_handle_factory):
     D = R @ G.T
     assert not np.any(np.abs(D) <= 1e-12 * np.linalg.norm(R, axis=1)[:, None] * np.linalg.norm(G, axis=1)[None, :])
     check_against_reference(res, C, start_vectors(R, G), 1000)
-
-
-def _gpus():
-    try:
-        import torch
-        return torch.cuda.device_count() if torch.cuda.is_available() else 0
-    except Exception:
-        return 0
-
-
-@pytest.mark.parametrize("world", [2, 4, 8])
-def test_local_search_on_several_gpus(world):
-    if _gpus() < world:
-        pytest.skip(f"needs {world} GPUs on one node (have {_gpus()})")
-    from test_gpu_multi import _torchrun
-    out = _torchrun(world, "check_multigpu_local_search.py", 29680 + world)
-    tail = out.stdout[-3000:] + "\n" + out.stderr[-3000:]
-    assert out.returncode == 0 and "MULTIGPU LOCAL SEARCH OK" in out.stdout, tail

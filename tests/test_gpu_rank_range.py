@@ -16,8 +16,7 @@ import scipy.sparse as sps
 
 from conftest import GPU_CONFIG_PARAMS
 from helpers import dense_S, g1_graph
-from test_gpu_local_search import check_against_reference, start_vectors
-from test_gpu_rounding import check_exact
+from rounding_reference import check_against_reference, check_exact, start_vectors
 
 pytestmark = pytest.mark.gpu
 

@@ -7,43 +7,13 @@ import scipy.sparse as sps
 
 from conftest import GPU_CONFIG_PARAMS
 from helpers import COMBOS, families, g1_graph, make_case
+from rounding_reference import check_exact, numpy_rounding
 
 pytestmark = pytest.mark.gpu
 
 
-def numpy_rounding(R, G, C):
-    """x_k = sign(R g_k) (ties to +1), obj_k = x_k' C x_k, sum_k; plus the candidates with a dot inside a 1e-12 relative
-    margin of zero (their sign is not determined by the data)."""
-    D = R @ G.T
-    X = np.where(D >= 0, 1.0, -1.0)
-    scale = np.linalg.norm(R, axis=1)[:, None] * np.linalg.norm(G, axis=1)[None, :]
-    ambiguous = np.any(np.abs(D) <= 1e-12 * scale, axis=0) & np.any(scale > 0, axis=0)
-    obj = np.einsum("ik,ik->k", X, sps.csr_matrix(C) @ X)
-    return X, obj, X.sum(axis=0), ambiguous
-
-
-def cut_value(A, x):
-    Au = sps.triu(sps.csr_matrix(A), k=1).tocoo()
-    return float(np.sum(Au.data * (x[Au.row] != x[Au.col])))
-
-
 def engine_for(sp, gpu_handle_factory, config, C, As, bs):
     return sp.B200Engine(sp.SDPData(C, As, bs), handle=gpu_handle_factory(config))
-
-
-def check_exact(res, R, G, C, A=None):
-    X, obj, tot, amb = numpy_rounding(R, G, C)
-    assert not amb.any(), f"{int(amb.sum())} candidates with a row inside the tie margin"
-    np.testing.assert_array_equal(res["G_used"], G)
-    np.testing.assert_array_equal(res["obj"], obj)
-    np.testing.assert_array_equal(res["sum"], tot)
-    b = res["best"]
-    assert b == int(np.argmin(obj))
-    np.testing.assert_array_equal(res["best_x"], X[:, b])
-    if A is not None:
-        for k in range(G.shape[0]):
-            assert res["obj"][k] == -cut_value(A, X[:, k])
-    return X
 
 
 @pytest.mark.parametrize("config", GPU_CONFIG_PARAMS)
@@ -232,9 +202,12 @@ def _gpus():
 
 @pytest.mark.parametrize("world", [2, 4, 8])
 def test_rounding_on_several_gpus(world):
+    """hyperplane rounding, local search and sweep rounding on 2 / 4 / 8 ranks, every rank exact against NumPy"""
     if _gpus() < world:
         pytest.skip(f"needs {world} GPUs on one node (have {_gpus()})")
     from test_gpu_multi import _torchrun
     out = _torchrun(world, "check_multigpu_rounding.py", 29660 + world)
     tail = out.stdout[-3000:] + "\n" + out.stderr[-3000:]
-    assert out.returncode == 0 and "MULTIGPU ROUNDING OK" in out.stdout, tail
+    assert out.returncode == 0, tail
+    for method in ("ROUNDING", "LOCAL SEARCH", "SWEEP"):
+        assert f"MULTIGPU {method} OK" in out.stdout, tail

@@ -10,63 +10,9 @@ import scipy.sparse as sps
 
 from conftest import GPU_CONFIG_PARAMS
 from helpers import g1_graph, make_case
+from rounding_reference import INF, assert_order_determined, cut_value, engine_with_R, numpy_sweep, projections
 
 pytestmark = pytest.mark.gpu
-
-INF = math.inf
-
-
-def projections(R, G):
-    """P = R G' computed once per distinct row of R, so exactly repeated rows get exactly equal projections (as on the
-    device, where a row's projection depends only on the row)"""
-    U, inv = np.unique(R, axis=0, return_inverse=True)
-    return (U @ G.T)[inv.reshape(-1)]
-
-
-def assert_order_determined(R, G, P):
-    """no two vertices adjacent in a sweep order (and no vertex at 0) lie within a 1e-12 relative margin unless their rows
-    of R are identical: the order and the hyperplane bits are then fixed by the data, not by the summation order"""
-    scale = np.linalg.norm(R, axis=1)[:, None] * np.linalg.norm(G, axis=1)[None, :]
-    _, rid = np.unique(R, axis=0, return_inverse=True)
-    rid = rid.reshape(-1)
-    for k in range(G.shape[0]):
-        p, sc = P[:, k], scale[:, k]
-        o = np.lexsort((np.arange(len(p)), p))
-        gap = np.abs(np.diff(p[o]))
-        close = (gap <= 1e-12 * np.maximum(sc[o][1:], sc[o][:-1])) & (rid[o][1:] != rid[o][:-1])
-        assert not close.any(), f"candidate {k}: {int(close.sum())} adjacent projections inside the tie margin"
-        assert not np.any((np.abs(p) <= 1e-12 * sc) & (p != 0.0)), f"candidate {k}: a projection inside the margin of 0"
-
-
-def numpy_sweep(C, P, w=None, window=(-INF, INF)):
-    """per candidate: order, profile f(0..n), W(S_0..n), chosen t (-1 if none feasible), x and obj of the chosen vector"""
-    Cs = sps.csr_matrix(C)
-    n, K = P.shape
-    A = Cs.copy()
-    A.setdiag(0.0)
-    A.eliminate_zeros()
-    coo = A.tocoo()
-    rows, cols, vals = coo.row, coo.col, coo.data
-    total = float(Cs.sum())
-    wv = np.ones(n) if w is None else np.asarray(w, dtype=np.float64)
-    out = []
-    for k in range(K):
-        order = np.lexsort((np.arange(n), P[:, k]))
-        pos = np.empty(n, np.int64)
-        pos[order] = np.arange(n)
-        s = np.where(pos[cols] > pos[rows], 1.0, -1.0)          # +1: the neighbour comes after the vertex
-        delta = -4.0 * np.bincount(rows, weights=vals * s, minlength=n)
-        prof = total + np.concatenate([[0.0], np.cumsum(delta[order])])
-        W = np.concatenate([[0.0], np.cumsum(wv[order])])
-        feas = (window[0] <= W) & (W <= window[1])
-        t = int(np.argmin(np.where(feas, prof, INF))) if feas.any() else -1
-        x = np.ones(n)
-        if t >= 0:
-            x[order[:t]] = -1.0
-        obj = float(x @ (Cs @ x)) if t >= 0 else INF
-        out.append({"order": order, "profile": prof, "W": W, "t": t, "x": x, "obj": obj})
-    return out
-
 
 def check_exact(res, ref, n):
     thresh = np.array([c["t"] for c in ref])
@@ -81,12 +27,6 @@ def check_exact(res, ref, n):
     np.testing.assert_array_equal(res["best_x"], ref[b]["x"])
     np.testing.assert_array_equal(res["best_order"], ref[b]["order"])
     np.testing.assert_array_equal(res["best_profile"], ref[b]["profile"])
-
-
-def engine_with_R(sp, gpu_handle_factory, config, data, R):
-    eng = sp.B200Engine(data, handle=gpu_handle_factory(config))
-    eng.init_vars(R.shape[1], R, np.zeros(data.m), 2.0, 4)
-    return eng
 
 
 def check_maxcut(eng, R, C, K=40, seed=None, G=None):
@@ -123,11 +63,6 @@ def test_maxcut_g1_exact(sp, gpu_handle_factory, config):
     assert out["obj"] <= hp["obj"]
     assert float(out["x"] @ (sps.csr_matrix(C) @ out["x"])) == out["obj"]
     ans["engine"].close()
-
-
-def cut_value(A, x):
-    Au = sps.triu(sps.csr_matrix(A), k=1).tocoo()
-    return float(np.sum(Au.data * (x[Au.row] != x[Au.col])))
 
 
 @pytest.mark.parametrize("drop", [False, True])
@@ -304,21 +239,3 @@ def test_argument_errors(sp, gpu_handle_factory):
         eng.round_sweep(8)
     assert e.value.code == -2
     eng.close()
-
-
-def _gpus():
-    try:
-        import torch
-        return torch.cuda.device_count() if torch.cuda.is_available() else 0
-    except Exception:
-        return 0
-
-
-@pytest.mark.parametrize("world", [2, 4, 8])
-def test_sweep_on_several_gpus(world):
-    if _gpus() < world:
-        pytest.skip(f"needs {world} GPUs on one node (have {_gpus()})")
-    from test_gpu_multi import _torchrun
-    out = _torchrun(world, "check_multigpu_sweep.py", 29700 + world)
-    tail = out.stdout[-3000:] + "\n" + out.stderr[-3000:]
-    assert out.returncode == 0 and "MULTIGPU SWEEP OK" in out.stdout, tail
